@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — particle-steps/s of the SPH step engine on synthetic Keplerian-disc ICs (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--particles P] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--particles P] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one body of the reference loop (SUMMER_SPH - Variable.f90:1120-1162): two full evaluations
 (tree + density + EOS + gravity + sinks + SPH pairs), two half kicks, drift, dt ladder, h Newton-Raphson,
@@ -12,6 +12,10 @@ version banner on stdout once when the first communicator of a multi-rank run is
 
 --impl reference times the CPU implementation of the same path (the oracle port of the Fortran loops —
 no Fortran compiler exists in this image, so the reference itself cannot be built) on the host cores.
+
+--dump-outputs DIR writes the state the last timed step handed back (what sph_download gives a caller) to DIR as
+float64 .npy files: the ten gas columns on a fixed, seeded sample of rows, every sink, dt and t.  The ICs come from a
+fixed seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -23,6 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: the benchmark leaves nothing in it
 
 import numpy as np  # noqa: E402
 
@@ -88,7 +93,7 @@ def make_ics(n):
     return b, s
 
 
-def cpu_reference_rate(n_sample, steps, warmup, threads):
+def cpu_reference_rate(n_sample, steps, warmup, threads, dump=None):
     """Oracle port timed on the host cores: particle-steps/s on a bounded disc sample."""
     from summersph_b200 import default_params, MODE_VARIABLE_H
     from oracle.oracle import Oracle
@@ -103,6 +108,8 @@ def cpu_reference_rate(n_sample, steps, warmup, threads):
     for _ in range(steps):
         dt, t = o.step(dt, t)
     el = time.perf_counter() - t0
+    if dump:
+        dump_outputs(dump, o, dt, t, 0)
     n, _ = o.sizes()
     return n * steps / el, el / steps
 
@@ -115,7 +122,7 @@ def run_reference(args, rank):
         return
     threads = min(REF_THREADS, os.cpu_count() or 1)
     n_sample = args.ref_particles
-    rate, sec = cpu_reference_rate(n_sample, args.steps, args.warmup, threads)
+    rate, sec = cpu_reference_rate(n_sample, args.steps, args.warmup, threads, dump=args.dump_outputs)
     line = {
         "impl": "reference", "metric": "particle-steps/s", "value": rate, "unit": "particle-steps/s", "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "strong",
@@ -196,6 +203,27 @@ def timed_run(e, n, steps, warmup, barrier, sampler=None, before=None):
     return ms, stage_acc, e.launch_count() - l0, clocks, (dt, t)
 
 
+DUMP_ROWS = 1 << 19          # sampled gas rows: 10 FP64 columns of them (40 MB) + their row numbers + the sinks stay under 64 MB
+DUMP_SEED = 20251018
+
+
+def dump_outputs(directory, e, dt, t, rank):
+    """--dump-outputs: the state after the last timed step as float64 DIR/<name>.npy.  Gas columns on DUMP_ROWS rows drawn
+    with a fixed seed (all rows when there are fewer; `rows` holds the row numbers), sink_<column> for every sink, dt_t."""
+    from summersph_b200.state import GAS_FIELDS, SINK_FIELDS
+    b, s = e.download()                          # under the domain decomposition a collective: every rank takes part
+    if rank != 0:
+        return
+    n = len(b)
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+    out = {"rows": rows, "dt_t": np.array([dt, t])}
+    out.update({k: getattr(b, k)[rows] for k in GAS_FIELDS})
+    out.update({"sink_" + k: getattr(s, k) for k in SINK_FIELDS})
+    os.makedirs(directory, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(directory, k + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -213,6 +241,7 @@ def main():
     ap.add_argument("--no-check", action="store_true", help="skip the untimed multi-rank vs single-rank comparison")
     ap.add_argument("--drift", action="store_true", help="add the energy / momentum / angular-momentum drift over the timed steps "
                     "(sph_conserved before and after them, outside the timed region) as a \"drift\" key (single rank / replicated form)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state after the last timed step to DIR/<name>.npy (float64; gas rows sampled with a fixed seed)")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -295,6 +324,8 @@ def main():
     dstats = e.domain_stats()
     dstats_all = {k: [int(x) for x in allgather(float(dstats[k]))] for k in ("own", "halo", "let_nodes")} if decomp else None
     state_hash, state_sums = e.state_hash()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, e, dt, t, rank)
     drift = None
     if want_drift:
         from summersph_b200._abi import drift_report
