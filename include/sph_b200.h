@@ -288,7 +288,10 @@ int sph_fp64_peak(sph_ctx* ctx, double* tflops);
  *           derivative is the reference's g(q)/q^2 (F:91,94); i's own single-particle leaf is left out
  *   out[11] sink terms: -G m_s m_j / r over sink-gas and sink-sink pairs (unsoftened like F:559-591)
  * n_out <= SPH_CONSERVED_COUNT slots are written.  Builds the octree of the current positions if the context
- * holds none (it is then reused by the next evaluation); in a multi-GPU run every rank returns the same sums. */
+ * holds none (it is then reused by the next evaluation); in a multi-GPU run every rank returns the same sums.
+ * Under decomposition = 1 the call is collective (every rank calls it; the build then includes migration, halo and
+ * locally essential tree); every rank returns the same values, equal to the single-rank sums up to rounding (the sum
+ * over particles is grouped by rank), not bit for bit. */
 #define SPH_CONSERVED_COUNT 12
 int sph_conserved(sph_ctx* ctx, double* out, int32_t n_out);
 
@@ -305,7 +308,9 @@ int sph_download_sink_spin(sph_ctx* ctx, double* spin_x, double* spin_y, double*
  *   image[iv * nu + iu] = sum_j m_j F(|d| / h_j) / (pi h_j^2),  d = pixel centre - particle in the image plane,
  * F = line-of-sight integral of the M4 kernel shape (F:66,70).  axis = 0|1|2 projects along x|y|z with image
  * axes (y,z)|(z,x)|(x,y); pixel (iu, iv) is centred at (u0 + (iu+1/2)(u1-u0)/nu, v0 + (iv+1/2)(v1-v0)/nv).
- * Particles narrower than a pixel are widened to h = pixel/2.  `image` holds nu*nv doubles (host memory). */
+ * Particles narrower than a pixel are widened to h = pixel/2.  `image` holds nu*nv doubles (host memory).
+ * Under decomposition = 1 the call is collective: every rank scatters the particles it owns and the images are
+ * summed over the ranks; every rank returns the same image, equal to the single-rank one up to rounding. */
 int sph_column_density(sph_ctx* ctx, int32_t axis, double u0, double u1, double v0, double v1,
                        int32_t nu, int32_t nv, double* image);
 

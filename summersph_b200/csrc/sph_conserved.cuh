@@ -12,8 +12,8 @@
 //             g(q) / q^2 (the polynomials of init_grav_kernel_table, F:91,94), -1/q beyond q = 2.
 //   E_sink  = -G sum_sinks sum_gas m_s m_j / r  -  G sum_{sink pairs} m_a m_b / r     (unsoftened, F:559-591)
 //   P, L    = sum m v, sum m x cross v over gas and sinks (+ the sinks' spin when SPH_FLAG_SINK_MERGE_SPIN keeps it); M = total mass.
-// The walk here is one thread per particle over the preorder octree with skip pointers (GNode.next): a diagnostic
-// called a few times per run, not a hot kernel.
+// The walk is one thread per particle over the gravity walk layout (WNode): a diagnostic called a few times per run,
+// not a hot kernel.
 #pragma once
 #include "sph_common.cuh"
 #include "sph_integrate.cuh"
@@ -36,9 +36,35 @@ __host__ __device__ inline double soft_potential(double q) {
   return -1.0 / q;
 }
 
-__global__ void __launch_bounds__(CONS_THREADS)
-k_conserved_partial(int n, int n_nodes, DevParams P, StateArrays s, const GNode* __restrict__ nodes,
-                    const int* __restrict__ node_part, int n_sink, SinkArrays S, double* __restrict__ partial) {
+// Row of the particle of every single-particle leaf of the local tree in the walk layout, -1 for every other slot
+// (internal and depth-limited childless nodes).  Rows, not numbers: what the walk leaves out is the particle itself,
+// whatever numbers the host gave the rows.  wbase: first slot of the local tree (0; DD_TOP_CAP under domains).
+__global__ void k_conserved_wpart(int n_nodes, const int* __restrict__ node_part, const int* __restrict__ widx, int wbase,
+                                  int* __restrict__ wpart) {
+  const int v = blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= n_nodes) return;
+  const int w = widx[v];
+  if (w >= 0) wpart[wbase + w] = node_part[v] >= 0 ? node_part[v] : -1;
+}
+
+// Walk layout: root at slot 0, the children of a node at [child, child + nchild), nchild == 0 accepted whole (leaves and
+// depth-limited childless nodes, F:182).  Children are visited in block order, which is the octree's preorder
+// (k_oct_widx assigns each block in child-chain order), so every particle sums the nodes of the preorder walk with skip
+// pointers in the same order and with the same bits.  Under domains the layout is [top | local | LET]: top nodes are
+// assembled in k_oct_up's order and LET nodes are bit copies, so each particle's term equals its single-rank term.  A
+// LET node whose children were not pulled still holds the owner's child index; it is never opened here, because the
+// LET pulls the children of every node that passes dd_may_open (soft = 0 plus a margin against the domain's position
+// boxes), a superset of the nodes this test (soft > 0) opens.
+// wpart: k_conserved_wpart under the layout (plus the top slots that copy one of this rank's single-particle leaves;
+// -1 on the LET slots: a remote particle is never i).
+// Stack: one (cursor, end) pair per opened level; the pair being walked stays in registers and a level is pushed only
+// when siblings remain (so one pop always yields a node: every trip of the loop visits one).  A node is opened only
+// above lmax <= SPH_KEY_LEVELS2, so at most 42 pairs are stacked.  The walk is bound by the latency of its dependent node
+// loads: 8 resident blocks (64 registers, a few accumulator spills) walk as fast as the preorder walk did; at the
+// 80 registers the compiler picks by itself (6 blocks) the 16M call is 1.27x slower on a B200.
+__global__ void __launch_bounds__(CONS_THREADS, 8)
+k_conserved_partial(int n, DevParams P, StateArrays s, const WNode* __restrict__ wn, const int* __restrict__ wpart,
+                    int n_sink, SinkArrays S, double* __restrict__ partial) {
   double acc[CONS_SUMS];
 #pragma unroll
   for (int k = 0; k < CONS_SUMS; ++k) acc[k] = 0.0;
@@ -56,17 +82,23 @@ k_conserved_partial(int n, int n_nodes, DevParams P, StateArrays s, const GNode*
     const double inv_h = 1.0 / hi;
     const double soft = P.soft_hi ? 0.001 * hi : 0.001 * P.h_fixed;          // F:275 | V:296 | T:298
     double phi = 0.0;
-    int v = 0;
-    while (v < n_nodes) {
-      const GNode g = nodes[v];
+    int2 stk[SPH_KEY_LEVELS2];
+    int sp = 0, cur = 0, end = 1;                                              // the root block: slot 0 alone
+    for (;;) {
+      const int v = cur++;
+      const WNode g = wn[v];
       const double dx = xi - g.cx, dy = yi - g.cy, dz = zi - g.cz;
       const double d2 = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)), soft);   // F:275
       const double dist = __dsqrt_rn(d2);
-      if ((g.flags & 1) || __ddiv_rn(g.size, dist) < P.theta) {                // F:278
-        if (g.m > 0.0 && dist > 0.0 && node_part[v] != i) phi += g.m * (soft_potential(dist * inv_h) * inv_h);
-        v = g.next;
+      if (g.nchild == 0 || __ddiv_rn(g.size, dist) < P.theta) {                // F:278
+        if (g.m > 0.0 && dist > 0.0 && wpart[v] != i) phi += g.m * (soft_potential(dist * inv_h) * inv_h);
       } else {
-        v = v + 1;                                                             // first child in preorder
+        if (cur < end) stk[sp++] = make_int2(cur, end);
+        cur = g.child; end = g.child + g.nchild;
+      }
+      if (cur == end) {                                                        // block done: a stacked level always has siblings left
+        if (sp == 0) break;
+        --sp; cur = stk[sp].x; end = stk[sp].y;
       }
     }
     acc[9] += 0.5 * mi * (P.G * phi);
@@ -94,10 +126,8 @@ k_conserved_partial(int n, int n_nodes, DevParams P, StateArrays s, const GNode*
   }
 }
 
-// one warp: fold the block partials in block order, add the sinks' own terms, write the CONS_FIELDS outputs
-__global__ void k_conserved_final(int nblocks, const double* __restrict__ partial, DevParams P, int n_sink, SinkArrays S,
-                                  const double* __restrict__ spin, double* __restrict__ out) {
-  __shared__ double tot[CONS_SUMS];
+// one warp: the CONS_SUMS totals of `nblocks` partials (lane-strided, then a warp sum: a fixed order); lane 0 writes tot
+__device__ __forceinline__ void cons_fold(int nblocks, const double* __restrict__ partial, double* tot) {
   const int l = threadIdx.x;
   for (int k = 0; k < CONS_SUMS; ++k) {
     double t = 0.0;
@@ -105,6 +135,18 @@ __global__ void k_conserved_final(int nblocks, const double* __restrict__ partia
     t = warp_sum(t);
     if (l == 0) tot[k] = t;
   }
+}
+
+// domains: one rank's CONS_SUMS totals (all-gathered, then folded by k_conserved_final like block partials)
+__global__ void k_conserved_fold(int nblocks, const double* __restrict__ partial, double* __restrict__ out) { cons_fold(nblocks, partial, out); }
+
+// one warp: fold the block partials (or, under domains, the ranks' totals), add the sinks' own terms once, write the
+// CONS_FIELDS outputs
+__global__ void k_conserved_final(int nblocks, const double* __restrict__ partial, DevParams P, int n_sink, SinkArrays S,
+                                  const double* __restrict__ spin, double* __restrict__ out) {
+  __shared__ double tot[CONS_SUMS];
+  const int l = threadIdx.x;
+  cons_fold(nblocks, partial, tot);
   __syncwarp();
   if (l != 0) return;
   double ekin = tot[0], px = tot[2], py = tot[3], pz = tot[4], lx = tot[5], ly = tot[6], lz = tot[7], mass = tot[8];

@@ -110,7 +110,7 @@ __global__ void k_dd_migrate(const __grid_constant__ DDMigrate a) {
 
 // ---- top tree: locally complete children of the cells that straddle a domain boundary ---------------------------------
 struct DDCell { uint64_t prefix; int level; int child_top; };    // child_top bit c: child octant c straddles too (is a top cell itself)
-struct DDContrib { double m, sx, sy, sz, size; int count, nchild, child, pad; };
+struct DDContrib { double m, sx, sy, sz, size; int count, nchild, child, row; };      // row: the particle's local row when count == 1, else -1
 // one thread per (cell, octant): if the child cell is not a top cell and holds particles of THIS rank, the rank owns all
 // of it: report its node (pre-finalize sums, so the top nodes add children exactly like k_oct_up does)
 __global__ void k_dd_top_contrib(int ncell, const DDCell* __restrict__ cells, int n, const uint64_t* __restrict__ key,
@@ -119,7 +119,7 @@ __global__ void k_dd_top_contrib(int ncell, const DDCell* __restrict__ cells, in
                                  DDContrib* __restrict__ out, int* err_flag) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= ncell * 8) return;
-  DDContrib rec; rec.m = rec.sx = rec.sy = rec.sz = rec.size = 0.0; rec.count = rec.nchild = rec.child = rec.pad = 0;
+  DDContrib rec; rec.m = rec.sx = rec.sy = rec.sz = rec.size = 0.0; rec.count = rec.nchild = rec.child = 0; rec.row = -1;
   const DDCell C = cells[t >> 3]; const int c = t & 7;
   if (!((C.child_top >> c) & 1) && n > 0 && C.level < SPH_KEY_LEVELS) {
     const int shift = 3 * (SPH_KEY_LEVELS - 1 - C.level);
@@ -137,7 +137,7 @@ __global__ void k_dd_top_contrib(int ncell, const DDCell* __restrict__ cells, in
       else {
         const GNode g = nodes[v];
         rec.m = g.m; rec.sx = g.cx; rec.sy = g.cy; rec.sz = g.cz; rec.size = g.size;
-        rec.count = b - a + 1; rec.nchild = wcount[v]; rec.child = 1 + wstart[v];
+        rec.count = b - a + 1; rec.nchild = wcount[v]; rec.child = 1 + wstart[v]; rec.row = a == b ? a : -1;
       }
     }
   }

@@ -101,7 +101,8 @@ struct sph_ctx {
   std::vector<std::vector<double*>> peer;      // [array slot][rank]
   std::vector<void*> ipc_opened; int* d_flag = nullptr; void* d_blob = nullptr; size_t blob_cap = 0;
   int g0 = 0, g1 = 0, p0 = 0, p1 = 0;
-  double* cons_partial = nullptr; double* cons_out = nullptr;   // sph_conserved: block partials, result slots
+  double* cons_partial = nullptr; double* cons_out = nullptr;   // sph_conserved: block partials (+ the ranks' totals under domains), result slots
+  int* cons_wpart = nullptr; size_t cons_wpart_n = 0;            // sph_conserved: per walk-layout slot, the row of a single-particle leaf (else -1)
   // far-field reuse of the gravity walk (sph_gravity.cuh): stored far sums of the tree terms, per-particle near / far split, the walk's counters
   double *far_fx = nullptr, *far_fy = nullptr, *far_fz = nullptr, *far_hc2 = nullptr; unsigned long long* far_ctr = nullptr;
   bool far_valid = false; int far_reuse = 1; int64_t far_count = 0; bool far_want_store = false; int steps_since_upload = 0; double far_hcut = GW_HCUT;
@@ -117,7 +118,7 @@ struct sph_ctx {
   // ---- Morton-domain decomposition (sph_domain.cuh / sph_domain_host.inl); in this mode n = own particles, cap = own + halo capacity
   bool dd = false; int64_t n_global = 0; int n_halo = 0, ng_own = 0, ng_halo = 0;
   uint64_t* key_alloc[2] = {}; int* perm_alloc[2] = {};          // the allocations behind key[] / perm[] (which swap)
-  uint64_t *dd_samples = nullptr, *dd_split = nullptr; long long* dd_counts = nullptr; int* dd_sendoff = nullptr; uint64_t* dd_segkeys = nullptr; std::vector<WNode> dd_top_host;
+  uint64_t *dd_samples = nullptr, *dd_split = nullptr; long long* dd_counts = nullptr; int* dd_sendoff = nullptr; uint64_t* dd_segkeys = nullptr; std::vector<WNode> dd_top_host; std::vector<int> dd_top_part;
   DDCell* dd_cells = nullptr; DDContrib* dd_contrib = nullptr; BvhBox* dd_obvh = nullptr; size_t dd_obvh_cap = 0; DDBvh dd_ob; int* dd_let_ctl = nullptr; double* dd_create8 = nullptr; unsigned long long* dd_cand = nullptr;
   bool dd_fields_pending = false; cudaEvent_t let_done = nullptr; bool let_pending = false; double* let_flag = nullptr; std::vector<DDLetEntry> dd_cand_host;
   DDLetEntry* dd_let_f[2] = {}; int dd_let_fcap = 0, dd_let_begin = 0, dd_let_end = 0, dd_let_used = 0, dd_top_n = 0;
@@ -1216,7 +1217,7 @@ int sph_destroy(sph_ctx* c) {
   F(c->dd_samples); F(c->dd_split); F(c->dd_counts); F(c->dd_sendoff); F(c->dd_segkeys); F(c->dd_cells); F(c->dd_contrib); F(c->dd_obvh); F(c->dd_let_ctl); F(c->dd_create8); F(c->dd_cand);
   F(c->dd_let_f[0]); F(c->dd_let_f[1]); F(c->dd_halo_flag); F(c->dd_halo_list); F(c->dd_halo_size); F(c->dd_halo_poff); F(c->dd_acc_key); F(c->dd_acc_rec);
   F(c->dd_accg_key[0]); F(c->dd_accg_key[1]); F(c->dd_accg_idx[0]); F(c->dd_accg_idx[1]); F(c->dd_accg_rec); F(c->dd_gid); F(c->dd_gpos); F(c->dd_gcnt); F(c->dd_goff); F(c->dd_gstage);
-  F(c->cons_partial); F(c->cons_out); F(c->img_table); F(c->sink_spin);
+  F(c->cons_partial); F(c->cons_out); F(c->cons_wpart); F(c->img_table); F(c->sink_spin);
   F(c->far_fx); F(c->far_fy); F(c->far_fz); F(c->far_hc2); F(c->far_ctr); F(c->far_list); F(c->far_cnt); F(c->far_ovf); F(c->d_same); F(c->sink_land);
   F(c->arrive); F(c->cnt); F(c->off); F(c->root); F(c->partial); F(c->cub_tmp); F(c->d_wt); F(c->d_dwt); F(c->d_gt);
   F(c->sink_buf); F(c->sink_partial); F(c->sink_seg); F(c->sc); F(c->ctr); F(c->work); F(c->keep); F(c->d_nsel); F(c->pos); F(c->stage_d); F(c->stage_d2);
@@ -1867,19 +1868,41 @@ int sph_fp64_peak(sph_ctx* c, double* tflops) {
 
 int sph_conserved(sph_ctx* c, double* out, int32_t n_out) {
   if (!c || !out || n_out < 1) return SPH_ERR_ARG;
-  if (c->n < 2) { c->err = "need at least 2 gas particles"; return SPH_ERR_STATE; }
-  if (c->dd) { c->err = "sph_conserved is not available under the domain decomposition (use decomposition = 0 for the drift report)"; return SPH_ERR_STATE; }
+  if ((c->dd ? c->n_global : c->n) < 2) { c->err = "need at least 2 gas particles"; return SPH_ERR_STATE; }
   cudaSetDevice(c->device);
   double keep_ms[ST_COUNT]; std::memcpy(keep_ms, c->stage_ms, sizeof(keep_ms));
-  if (!(c->tree_valid && !c->pos_moved)) {        // the octree of the current positions (kept for the next evaluation)
+  if (!(c->tree_valid && !c->pos_moved)) {        // the octree of the current positions (kept for the next evaluation); domains: migration, halo, LET
     int r = build_tree(c); if (r) return r;
   }
-  if (!c->cons_partial) { DA(c->cons_partial, (size_t)CONS_MAX_BLOCKS * CONS_SUMS); DA(c->cons_out, CONS_FIELDS); }
+  if (!c->cons_partial) { DA(c->cons_partial, (size_t)(CONS_MAX_BLOCKS + DD_MAX_RANKS) * CONS_SUMS); DA(c->cons_out, CONS_FIELDS); }
+  const size_t nslot = c->dd ? (size_t)c->dd_let_end : (size_t)(2 * c->cap);
+  if (nslot > c->cons_wpart_n) { c->cons_wpart_n = 0; DA(c->cons_wpart, nslot); c->cons_wpart_n = nslot; }
+  const int nn = (int)c->counts.n_nodes, T = 256;
+  if (c->dd) {
+    CK(cudaMemsetAsync(c->cons_wpart, 0xff, nslot * sizeof(int), c->stream));
+    CK(cudaMemcpyAsync(c->cons_wpart, c->dd_top_part.data(), c->dd_top_part.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+  }
+  LAUNCH(k_conserved_wpart, cdiv(nn, T), T, 0, nn, c->node_part, c->widx, c->dd ? DD_TOP_CAP : 0, c->cons_wpart);
+  if (c->dd) {      // the walk reads the LET: every rank's must be complete, and no rank may stop alone
+    if (c->let_pending) { CK(cudaStreamWaitEvent(c->stream, c->let_done, 0)); c->let_pending = false; }
+    double let_overflow = 0.0;
+    CK(cudaMemcpyAsync(&let_overflow, c->let_flag, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaMemcpyAsync(c->h_sc, c->sc, sizeof(SimScalars), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    int code = check_device_error(c);
+    if (!code && let_overflow > 0.0) { c->err = "domain decomposition: the locally essential tree of some rank exceeds its capacity (raise SPH_B200_DOMAIN_SLACK)"; code = SPH_ERR_OOM; }
+    { int r = dd_agree(c, code, "sph_conserved"); if (r) return r; }
+  }
   const int n = (int)c->n;
   const int nb = std::max(1, std::min(cdiv(n, CONS_THREADS), std::min(CONS_MAX_BLOCKS, c->n_sm * 16)));
-  LAUNCH(k_conserved_partial, nb, CONS_THREADS, 0, n, (int)c->counts.n_nodes, c->dp, state_of(c, c->cur), c->nodes, c->node_part,
-         c->n_sink, c->S, c->cons_partial);
-  LAUNCH(k_conserved_final, 1, 32, 0, nb, c->cons_partial, c->dp, c->n_sink, c->S, c->sink_spin, c->cons_out);
+  LAUNCH(k_conserved_partial, nb, CONS_THREADS, 0, n, c->dp, state_of(c, c->cur), c->wnodes, c->cons_wpart, c->n_sink, c->S, c->cons_partial);
+  if (c->dd) {      // each rank's totals, all-gathered and folded in rank order: every rank returns the same bits; the sinks are added once
+    double* rank_sums = c->cons_partial + (size_t)CONS_MAX_BLOCKS * CONS_SUMS;
+    LAUNCH(k_conserved_fold, 1, 32, 0, nb, c->cons_partial, rank_sums + (size_t)c->rank * CONS_SUMS);
+    { int r = coll_allgather(c, c->stream, rank_sums + (size_t)c->rank * CONS_SUMS, rank_sums, CONS_SUMS * sizeof(double)); if (r) return r; }
+    LAUNCH(k_conserved_final, 1, 32, 0, c->n_ranks, rank_sums, c->dp, c->n_sink, c->S, c->sink_spin, c->cons_out);
+  } else
+    LAUNCH(k_conserved_final, 1, 32, 0, nb, c->cons_partial, c->dp, c->n_sink, c->S, c->sink_spin, c->cons_out);
   double host[CONS_FIELDS];
   CK(cudaMemcpyAsync(host, c->cons_out, sizeof(host), cudaMemcpyDeviceToHost, c->stream));
   CK(cudaMemcpyAsync(c->h_sc, c->sc, sizeof(SimScalars), cudaMemcpyDeviceToHost, c->stream));
@@ -1895,8 +1918,9 @@ int sph_conserved(sph_ctx* c, double* out, int32_t n_out) {
 int sph_column_density(sph_ctx* c, int32_t axis, double u0, double u1, double v0, double v1, int32_t nu, int32_t nv, double* image) {
   if (!c || !image) return SPH_ERR_ARG;
   if (axis < 0 || axis > 2 || nu < 1 || nv < 1 || nu > 16384 || nv > 16384 || !(u1 > u0) || !(v1 > v0)) { c->err = "bad image frame"; return SPH_ERR_ARG; }
-  if (c->n <= 0) { c->err = "no particles uploaded"; return SPH_ERR_STATE; }
+  if ((c->dd ? c->n_global : c->n) <= 0) { c->err = "no particles uploaded"; return SPH_ERR_STATE; }
   cudaSetDevice(c->device);
+  const bool reduce = c->dd && c->n_ranks > 1;      // domains: every rank scatters its own rows (never the halo copies), the images are summed
   if (!c->img_table) {
     // F(q_b) = 2 int_0^sqrt(4 - q_b^2) w(sqrt(q_b^2 + s^2)) ds, w = the M4 shape of F:66,70; composite Simpson, 4096 intervals
     std::vector<double> F(IMG_TABLE + 2, 0.0);
@@ -1913,18 +1937,27 @@ int sph_column_density(sph_ctx* c, int32_t axis, double u0, double u1, double v0
   }
   double* d_img = nullptr;
   const size_t npx = (size_t)nu * nv;
-  if (cudaMalloc((void**)&d_img, npx * 8) != cudaSuccess) { cudaGetLastError(); c->err = "cudaMalloc(image)"; return SPH_ERR_OOM; }
+  const bool got = cudaMalloc((void**)&d_img, npx * 8) == cudaSuccess;
+  if (!got) { cudaGetLastError(); d_img = nullptr; c->err = "cudaMalloc(image)"; }
+  if (reduce) { int r = dd_agree(c, got ? 0 : SPH_ERR_OOM, "sph_column_density"); if (r) { cudaFree(d_img); return r; } }
+  else if (!got) return SPH_ERR_OOM;
+  int r = SPH_OK;
   cudaError_t e = cudaMemsetAsync(d_img, 0, npx * 8, c->stream);
   if (e == cudaSuccess) {
     const int n = (int)c->n;
     const int grid = std::max(1, std::min(cdiv((int64_t)n * 32, IMG_THREADS), c->n_sm * 8));
     LAUNCH(k_column_density, grid, IMG_THREADS, 0, n, state_of(c, c->cur), c->dp.variable_h, c->dp.h_fixed, (int)axis, u0, v0,
            (u1 - u0) / nu, (v1 - v0) / nv, (int)nu, (int)nv, c->img_table, d_img);
-    e = cudaMemcpyAsync(image, d_img, npx * 8, cudaMemcpyDeviceToHost, c->stream);
+    if (reduce) {      // NCCL: one all-reduce; the host communicator's all-gather carries at most SPH_HC_SLOT bytes per rank
+      const size_t chunk = c->hc ? SPH_HC_SLOT / 8 : npx;
+      for (size_t o = 0; o < npx && r == SPH_OK; o += chunk) r = coll_allreduce(c, c->stream, d_img + o, std::min(chunk, npx - o), NC_FLOAT64, NC_SUM);
+    }
+    if (r == SPH_OK) e = cudaMemcpyAsync(image, d_img, npx * 8, cudaMemcpyDeviceToHost, c->stream);
   }
   if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
   if (e == cudaSuccess) e = cudaGetLastError();
   cudaFree(d_img);
+  if (r != SPH_OK) return r;
   if (e != cudaSuccess) { c->err = std::string("sph_column_density: ") + cudaGetErrorString(e); return SPH_ERR_CUDA; }
   return SPH_OK;
 }

@@ -18,7 +18,9 @@ def simulate(bodies: Bodies, sinks: Sinks, params: SphParams, engine=None, save_
     `drift`: pass a dict to get the run's conservation report (north_star: "energy/momentum drift reported
     over the full run"): the engine's conserved sums (`sph_conserved`) are taken before the first and after the
     last step, the dict receives `first`, `last` and the relative drifts, and two extra lines are logged.  The
-    reference itself prints nothing of the kind, so the default leaves its output untouched.
+    reference itself prints nothing of the kind, so the default leaves its output untouched.  `drift=` works on a
+    multi-rank engine of either form when every rank calls `simulate` (under the Morton domains `sph_conserved` is
+    collective); every rank then gets the same report.
     Returns (bodies, sinks, t, dt, steps)."""
     own = engine is None
     if own:
