@@ -314,6 +314,39 @@ int sph_download_sink_spin(sph_ctx* ctx, double* spin_x, double* spin_y, double*
 int sph_column_density(sph_ctx* ctx, int32_t axis, double u0, double u1, double v0, double v1,
                        int32_t nu, int32_t nv, double* image);
 
+/* The SPH interpolant of the resident gas at n_points caller-given points (px, py, pz: host arrays), computed on the
+ * device: the point-wise counterpart of the density grid Density_Image.py builds with a KD-tree (:105-141), for slices,
+ * profiles along a line and grids.  For a point x and the gas particles j (sinks are point masses, not SPH particles,
+ * and take no part):
+ *   W(r, h) = w_table(r / h) / (pi h^3), the engine's table-interpolated cubic spline with the density pass's
+ *             normalisation: fixed h: h = h_fixed for every j, pi = 3.14159265359 (F:125-126); variable h: h = h_j,
+ *             pi in single precision (V:139-140)
+ *   members of x = { j : |x - x_j| / h_j <= 2 }  (scatter form, each particle's own h; the leaf-box test of F:443 |
+ *             V:479 plays no part, so particles of a depth-limited multi-particle leaf are ordinary members; a particle
+ *             whose h is not finite and positive contributes nothing)
+ *   out[k * n_points + i], k = 0 .. n_out - 1 (n_out <= SPH_INTERP_COUNT):
+ *     0  rho(x) = sum m_j W(|x - x_j|, h_j)
+ *     1..3  v = sum m_j v_j W / rho(x),  4  u = sum m_j u_j W / rho(x),  5  alpha = sum m_j alpha_j W / rho(x)
+ *           (0 where rho(x) = 0)
+ *     6  the number of members, as a double
+ * Mass weights, not m_j / rho_j: the result is a function of the resident x m h v u alpha alone, whichever evaluation
+ * ran last (the stored rho_j is stale after calc_smoothing, V:1152).  In fixed-h mode rho at x = x_i is the density
+ * pass's rho_i up to summation order.
+ * SPH_ERR_ARG: a NULL pointer, n_out outside 1..SPH_INTERP_COUNT, n_points < 0 or a non-finite coordinate;
+ * SPH_ERR_STATE: no gas uploaded; n_points = 0 is a no-op.  Builds the tree of the current positions if the context
+ * holds none (kept for the next evaluation, like sph_conserved); the sources are found through a private BVH over the
+ * walk groups, so nothing a later step reads changes, and sph_stage_times still reports the last step.  Points are
+ * processed in chunks of 2^22 (scratch is bounded and kept by the context).  A call returns the same bits when repeated,
+ * and for a permutation of the points (within one chunk) the permuted output.
+ * Replicated multi-GPU form: every rank computes everything locally and returns the same bits.  Under
+ * decomposition = 1 the call is collective: every rank passes the same points (checked: count and a hash of the
+ * coordinate bits; a mismatch is SPH_ERR_ARG on every rank), each rank sums over the particles it owns, the 7 raw sums
+ * are added over the ranks (NCCL all-reduce or the host communicator) and divided after that, so every rank returns
+ * the same bits, equal to the single-rank result up to rounding. */
+#define SPH_INTERP_COUNT 7
+int sph_interpolate(sph_ctx* ctx, int64_t n_points, const double* px, const double* py, const double* pz,
+                    double* out, int32_t n_out);
+
 #ifdef __cplusplus
 }
 #endif

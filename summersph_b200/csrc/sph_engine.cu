@@ -26,6 +26,7 @@
 #include "sph_integrate.cuh"
 #include "sph_conserved.cuh"
 #include "sph_image.cuh"
+#include "sph_interp.cuh"
 #include "sph_domain.cuh"
 #include "sph_ics.cuh"
 
@@ -115,6 +116,10 @@ struct sph_ctx {
   double* io_stage[5] = {}; size_t io_stage_cap = 0; bool io_active = false; double* io_out[10] = {}; unsigned io_fetched = 0; bool io_busy = false;
   double* sink_spin = nullptr; int sink_extras = 0;               // SPH_FLAG_SINK_MERGE_SPIN: spin[3][SPH_MAX_SINKS]; null pointer into the kernels when off
   double* img_table = nullptr;
+  // sph_interpolate: the private BVH of the source balls (2 h_j of the current h) and the per-chunk query scratch, grown on demand
+  double* ip_reach = nullptr; size_t ip_reach_cap = 0; BvhBox* ip_bvh = nullptr; size_t ip_bvh_cap = 0; BvhInfo ip_bi;
+  double *ip_pts = nullptr, *ip_raw = nullptr, *ip_bpart = nullptr; uint64_t *ip_key[2] = {}, *ip_tie[2] = {}; int* ip_idx[2] = {}; RootBox* ip_rb = nullptr;
+  void* ip_cub = nullptr; size_t ip_cub_bytes = 0; size_t ip_cap = 0;
   // ---- Morton-domain decomposition (sph_domain.cuh / sph_domain_host.inl); in this mode n = own particles, cap = own + halo capacity
   bool dd = false; int64_t n_global = 0; int n_halo = 0, ng_own = 0, ng_halo = 0;
   uint64_t* key_alloc[2] = {}; int* perm_alloc[2] = {};          // the allocations behind key[] / perm[] (which swap)
@@ -1109,6 +1114,92 @@ bool load_nccl(sph_ctx* c) {
   return true;
 }
 
+// ---- sph_interpolate (sph_interp.cuh) ------------------------------------------------------------------------------
+size_t interp_smem(const sph_ctx* c) {
+  return (size_t)((c->p.nq + 1) + ((c->p.nq + 1) & 1)) * 8 + (size_t)INTERP_WARPS * (INTERP_WARP_DOUBLES * 8 + WALK_WS * 4);
+}
+
+// The per-chunk scratch for `cap` points: coordinates, the 7 raw columns, sort keys (double-buffered), bounding-box partials.
+int interp_scratch(sph_ctx* c, size_t cap) {
+  if (cap <= c->ip_cap) return SPH_OK;
+  c->ip_cap = 0;
+  DA(c->ip_pts, 3 * cap); DA(c->ip_raw, (size_t)SPH_INTERP_COUNT * cap);
+  for (int b = 0; b < 2; ++b) { DA(c->ip_key[b], cap); DA(c->ip_tie[b], cap); DA(c->ip_idx[b], cap); }
+  if (!c->ip_bpart) { DA(c->ip_bpart, (size_t)c->n_partial * 6); DA(c->ip_rb, 1); }
+  size_t bytes = 0;
+  cub::DoubleBuffer<uint64_t> dk(c->ip_key[0], c->ip_key[1]); cub::DoubleBuffer<int> dv(c->ip_idx[0], c->ip_idx[1]);
+  cub::DeviceRadixSort::SortPairs(nullptr, bytes, dk, dv, (int)cap, 0, 64, c->stream);
+  DA(c->ip_cub, bytes + 256); c->ip_cub_bytes = bytes + 256;
+  c->ip_cap = cap;
+  return SPH_OK;
+}
+
+// Private BVH over the source walk groups (domains: the own groups only) with reach boxes that bound |x - x_j| <= 2 h_j.
+int interp_bvh(sph_ctx* c, int ng, int n_src) {
+  const int T = 256;
+  if ((size_t)n_src > c->ip_reach_cap) { c->ip_reach_cap = 0; DA(c->ip_reach, (size_t)c->cap); c->ip_reach_cap = (size_t)c->cap; }
+  if ((size_t)ng + ng / 7 + 64 > c->ip_bvh_cap) { c->ip_bvh_cap = 0; const size_t cap = (size_t)(ng + ng / 7 + 64) * 5 / 4; DA(c->ip_bvh, cap); c->ip_bvh_cap = cap; }
+  BvhInfo& bi = c->ip_bi;
+  bi.nlev = 1; bi.off[0] = 0; bi.cnt[0] = ng;
+  if (ng == 0) return SPH_OK;
+  StateArrays s = state_of(c, c->cur);
+  LAUNCH(k_interp_reach, cdiv(n_src, T), T, 0, n_src, s.h, c->dp.variable_h, c->dp.h_fixed, c->ip_reach);
+  LAUNCH(k_bvh_leaf, cdiv((int64_t)ng * 32, T), T, 0, ng, c->groups, s.x, s.y, s.z, s.x, s.y, s.z, c->ip_reach, c->ip_bvh);
+  int cntl = ng, offl = 0, l = 0;
+  while (cntl > 32) {
+    const int np = cdiv(cntl, SPH_BVH_FAN);
+    bi.off[l + 1] = offl + cntl; bi.cnt[l + 1] = np;
+    LAUNCH(k_bvh_up, cdiv(np, T), T, 0, cntl, c->ip_bvh + offl, c->ip_bvh + offl + cntl);
+    offl += cntl; cntl = np; ++l;
+  }
+  bi.nlev = l + 1;
+  return SPH_OK;
+}
+
+// One chunk of points [off, off + nc): sort, walk, (domains) sum the ranks' raw columns, finish, copy out.
+int interp_chunk(sph_ctx* c, int64_t off, int nc, const double* px, const double* py, const double* pz, int64_t n_points,
+                 double* out, int n_out, bool reduce) {
+  const int T = 256;
+  const size_t cap = c->ip_cap;
+  double* pts = c->ip_pts;
+  const double* src[3] = {px, py, pz};
+  for (int k = 0; k < 3; ++k) CK(cudaMemcpyAsync(pts + (size_t)k * cap, src[k] + off, (size_t)nc * 8, cudaMemcpyHostToDevice, c->stream));
+  const int nb = std::min(cdiv(nc, T), c->n_partial);
+  LAUNCH(k_bbox_partial, nb, T, 0, nc, pts, pts + cap, pts + 2 * cap, c->ip_bpart);
+  LAUNCH(k_bbox_final, 1, 32, 0, nb, c->ip_bpart, c->ip_rb);
+  LAUNCH(k_interp_keys, cdiv(nc, T), T, 0, nc, pts, pts + cap, pts + 2 * cap, c->ip_rb, c->ip_key[0], c->ip_tie[0], c->ip_idx[0]);
+  int* perm;
+  {   // stable LSD order: by the tie hash, then by the Morton key
+    size_t bytes = c->ip_cub_bytes;
+    cub::DoubleBuffer<uint64_t> dt(c->ip_tie[0], c->ip_tie[1]); cub::DoubleBuffer<int> dv(c->ip_idx[0], c->ip_idx[1]);
+    CK(cub::DeviceRadixSort::SortPairs(c->ip_cub, bytes, dt, dv, nc, 0, 64, c->stream));
+    LAUNCH(k_gather_u64, cdiv(nc, T), T, 0, nc, dv.Current(), c->ip_key[0], c->ip_key[1]);
+    int* alt = dv.Current() == c->ip_idx[0] ? c->ip_idx[1] : c->ip_idx[0];
+    cub::DoubleBuffer<uint64_t> dk(c->ip_key[1], c->ip_key[0]); cub::DoubleBuffer<int> dp(dv.Current(), alt);
+    bytes = c->ip_cub_bytes;
+    CK(cub::DeviceRadixSort::SortPairs(c->ip_cub, bytes, dk, dp, nc, 0, 63, c->stream));
+    perm = dp.Current();
+  }
+  const int ng = c->ip_bi.cnt[0];
+  StateArrays s = state_of(c, c->cur);
+  InterpArrays A{s.x, s.y, s.z, s.vx, s.vy, s.vz, s.u, s.m, s.alpha, s.h, c->ip_reach};
+  double* raw = c->ip_raw;
+  if (ng > 0) {
+    const int runs = cdiv(nc, 32);
+    LAUNCH(k_interpolate, cdiv(runs, INTERP_WARPS), INTERP_WARPS * 32, interp_smem(c), nc, pts, pts + cap, pts + 2 * cap, perm,
+           c->groups, A, c->ip_bvh, c->ip_bi, c->d_wt, c->dp, raw);
+  } else CK(cudaMemsetAsync(raw, 0, (size_t)SPH_INTERP_COUNT * nc * 8, c->stream));      // a domain without particles adds zeros
+  if (reduce) {      // NCCL: one all-reduce; the host communicator's all-gather carries at most SPH_HC_SLOT bytes per rank
+    const size_t tot = (size_t)SPH_INTERP_COUNT * nc, chunk = c->hc ? SPH_HC_SLOT / 8 : tot;
+    for (size_t o = 0; o < tot; o += chunk) { int r = coll_allreduce(c, c->stream, raw + o, std::min(chunk, tot - o), NC_FLOAT64, NC_SUM); if (r) return r; }
+  }
+  LAUNCH(k_interp_finish, cdiv(nc, T), T, 0, nc, raw);
+  for (int k = 0; k < n_out; ++k)
+    CK(cudaMemcpyAsync(out + (size_t)k * n_points + off, raw + (size_t)k * nc, (size_t)nc * 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return SPH_OK;
+}
+
 }  // namespace
 
 // =====================================================================================================
@@ -1189,6 +1280,7 @@ int sph_create(const sph_params* p, int32_t device, sph_ctx** out) {
   cudaFuncSetAttribute(k_gravity<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gravity_smem(c, grav_warps(c)));
   cudaFuncSetAttribute(k_gravity_near, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gravity_smem(c, 0));
   cudaFuncSetAttribute(k_neighbours, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(k_interpolate, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)interp_smem(c));
   if (cudaGetLastError() != cudaSuccess) { c->err = "cudaFuncSetAttribute failed (was the library built for this GPU's architecture?)"; return fail(SPH_ERR_CUDA); }
   *out = c;
   return SPH_OK;
@@ -1218,6 +1310,8 @@ int sph_destroy(sph_ctx* c) {
   F(c->dd_let_f[0]); F(c->dd_let_f[1]); F(c->dd_halo_flag); F(c->dd_halo_list); F(c->dd_halo_size); F(c->dd_halo_poff); F(c->dd_acc_key); F(c->dd_acc_rec);
   F(c->dd_accg_key[0]); F(c->dd_accg_key[1]); F(c->dd_accg_idx[0]); F(c->dd_accg_idx[1]); F(c->dd_accg_rec); F(c->dd_gid); F(c->dd_gpos); F(c->dd_gcnt); F(c->dd_goff); F(c->dd_gstage);
   F(c->cons_partial); F(c->cons_out); F(c->cons_wpart); F(c->img_table); F(c->sink_spin);
+  F(c->ip_reach); F(c->ip_bvh); F(c->ip_pts); F(c->ip_raw); F(c->ip_bpart); F(c->ip_rb); F(c->ip_cub);
+  for (int b = 0; b < 2; ++b) { F(c->ip_key[b]); F(c->ip_tie[b]); F(c->ip_idx[b]); }
   F(c->far_fx); F(c->far_fy); F(c->far_fz); F(c->far_hc2); F(c->far_ctr); F(c->far_list); F(c->far_cnt); F(c->far_ovf); F(c->d_same); F(c->sink_land);
   F(c->arrive); F(c->cnt); F(c->off); F(c->root); F(c->partial); F(c->cub_tmp); F(c->d_wt); F(c->d_dwt); F(c->d_gt);
   F(c->sink_buf); F(c->sink_partial); F(c->sink_seg); F(c->sc); F(c->ctr); F(c->work); F(c->keep); F(c->d_nsel); F(c->pos); F(c->stage_d); F(c->stage_d2);
@@ -1959,6 +2053,58 @@ int sph_column_density(sph_ctx* c, int32_t axis, double u0, double u1, double v0
   cudaFree(d_img);
   if (r != SPH_OK) return r;
   if (e != cudaSuccess) { c->err = std::string("sph_column_density: ") + cudaGetErrorString(e); return SPH_ERR_CUDA; }
+  return SPH_OK;
+}
+
+int sph_interpolate(sph_ctx* c, int64_t n_points, const double* px, const double* py, const double* pz, double* out, int32_t n_out) {
+  if (!c) return SPH_ERR_ARG;
+  cudaSetDevice(c->device);
+  const bool coll = c->dd && c->n_ranks > 1;      // domains: every rank walks its own rows for the same points, the raw sums are added
+  std::string why;
+  if (!px || !py || !pz || !out) why = "null pointer";
+  else if (n_out < 1 || n_out > SPH_INTERP_COUNT) why = "n_out must be 1.." + std::to_string(SPH_INTERP_COUNT);
+  else if (n_points < 0) why = "n_points < 0";
+  uint64_t hash = 0;
+  if (why.empty()) {
+    const double* col[3] = {px, py, pz};
+    for (int64_t i = 0; i < n_points && why.empty(); ++i)
+      for (int k = 0; k < 3; ++k) {
+        const double v = col[k][i];
+        if (!std::isfinite(v)) { why = "non-finite coordinate"; break; }
+        if (coll) { uint64_t b; std::memcpy(&b, &v, 8); hash = mix64(hash ^ b); }
+      }
+  }
+  if (coll) {      // the ranks compare their points (count, coordinate-bit hash, n_out) and argument checks: any mismatch stops every rank
+    struct Fp { int64_t n; uint64_t h; int32_t n_out, bad; };
+    Fp mine = {n_points, hash, n_out, why.empty() ? 0 : 1}, all[DD_MAX_RANKS];
+    { int r = dd_allgather_host(c, &mine, sizeof(Fp), all); if (r) return r; }
+    for (int q = 0; q < c->n_ranks && why.empty(); ++q) {
+      if (all[q].bad) why = "rank " + std::to_string(q) + " passed invalid arguments";
+      else if (all[q].n != mine.n || all[q].h != mine.h || all[q].n_out != mine.n_out) why = "the ranks passed different points (the call is collective: every rank passes the same points)";
+    }
+  }
+  if (!why.empty()) { c->err = "sph_interpolate: " + why; return SPH_ERR_ARG; }
+  if ((c->dd ? c->n_global : c->n) <= 0) { c->err = "no particles uploaded"; return SPH_ERR_STATE; }
+  if (n_points == 0) return SPH_OK;
+  double keep_ms[ST_COUNT]; std::memcpy(keep_ms, c->stage_ms, sizeof(keep_ms));
+  if (!(c->tree_valid && !c->pos_moved)) {        // the walk groups of the current positions (kept for the next evaluation); domains: migration, halo, LET
+    int r = build_tree(c); if (r) return r;
+  }
+  int code = interp_bvh(c, c->dd ? c->ng_own : c->n_groups, (int)c->n);      // domains: the own groups, never the halo copies
+  if (!code) code = interp_scratch(c, (size_t)std::min<int64_t>(n_points, SPH_INTERP_CHUNK));
+  CK(cudaMemcpyAsync(c->h_sc, c->sc, sizeof(SimScalars), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  stage_collect(c, false);                        // a tree build here is not part of any step's stage times
+  std::memcpy(c->stage_ms, keep_ms, sizeof(keep_ms));
+  if (!code) code = check_device_error(c);        // key-depth error of a tree built here
+  if (coll) { int r = dd_agree(c, code, "sph_interpolate"); if (r) return r; }
+  else if (code) return code;
+  for (int64_t off = 0; off < n_points; off += SPH_INTERP_CHUNK) {      // the chunks depend on n_points only: the same on every rank
+    const int nc = (int)std::min<int64_t>(SPH_INTERP_CHUNK, n_points - off);
+    int r = interp_chunk(c, off, nc, px, py, pz, n_points, out, n_out, coll);
+    if (r) return r;
+  }
+  CK(cudaGetLastError());
   return SPH_OK;
 }
 

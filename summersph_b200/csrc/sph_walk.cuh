@@ -54,13 +54,15 @@ __device__ __forceinline__ bool box_overlap(const float* alo, const float* ahi, 
 //   void   stage(int slot, int j)                    // copy source j into tile slot
 //   int    filter_stage(int j, bool in_range, int tn), void shift(int rest)    // FUSED: both at once, 2-tile slots
 //   void   consume(int count)                        // all lanes process tile[0..count)
+// The target box `tgt` is the warp's own: a walk group's level-0 box (the overload below), or the box of any other 32
+// targets (sph_interp.cuh: a run of interpolation points).
 template <class OP>
-__device__ void neighbour_walk(OP& op, const int2* __restrict__ groups, int chunk, const BvhBox* __restrict__ box, const BvhInfo& bi,
+__device__ void neighbour_walk(OP& op, const BvhBox& tgt, const int2* __restrict__ groups, const BvhBox* __restrict__ box, const BvhInfo& bi,
                                unsigned* stack, unsigned* cq) {
   unsigned* tix = cq + WALK_CQ;          // particle indices of the tile being collected
   const int lane = threadIdx.x & 31;
   const unsigned lt = (1u << lane) - 1u;
-  const BvhBox g = box[bi.off[0] + chunk];
+  const BvhBox g = tgt;
   int sn = 0, qn = 0, qpos = 0, tn = 0;
 
   auto hit = [&](const BvhBox& b) -> bool {
@@ -159,6 +161,12 @@ __device__ void neighbour_walk(OP& op, const int2* __restrict__ groups, int chun
       if (exhausted && !pend_cnt) break;
     }
   }
+}
+// targets = walk group `chunk`
+template <class OP>
+__device__ __forceinline__ void neighbour_walk(OP& op, const int2* __restrict__ groups, int chunk, const BvhBox* __restrict__ box, const BvhInfo& bi,
+                                               unsigned* stack, unsigned* cq) {
+  neighbour_walk(op, box[bi.off[0] + chunk], groups, box, bi, stack, cq);
 }
 
 // Saved candidate lists.  The density pass walks the BVH with the symmetric (pair-loop) criterion and writes,

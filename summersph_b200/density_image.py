@@ -8,7 +8,9 @@ own smoothing lengths (`sph_column_density`), either from a live engine or from 
     python -m summersph_b200.density_image save275.txt --variable --size 100 --pixels 512 --out save275.pgm
 
 Writes a binary PGM (8-bit, log scale like a colour-mapped imshow of a disc) and, with --npy, the raw FP64 image.
-There is no CPU path: the projection runs in the CUDA engine.
+With --slice OFFSET the image is instead the density on the plane `axis = OFFSET` (a cross-section, what SPLASH-style
+slice plots show), sampled at the pixel centres with `sph_interpolate`.
+There is no CPU path: the projection and the interpolation run in the CUDA engine.
 """
 import argparse
 import numpy as np
@@ -19,6 +21,23 @@ from ._abi import default_params, MODE_FIXED_H, MODE_VARIABLE_H
 def column_density(engine, axis="z", size=100.0, pixels=512):
     """Square frame |u|,|v| < size (Density_Image.py:64), `pixels` x `pixels`."""
     return engine.column_density(axis, (-size, size, -size, size), (pixels, pixels))
+
+
+_FRAME_AXES = {"x": (1, 2), "y": (2, 0), "z": (0, 1)}       # image axes (u, v) of each view axis, as sph_column_density
+
+
+def density_slice(engine, axis="z", offset=0.0, size=100.0, pixels=512):
+    """Density on the plane `axis = offset` at the pixel centres of the frame of `column_density` (|u|,|v| < size,
+    `pixels` x `pixels`, rows along v): `sph_interpolate` column rho."""
+    ax = {0: "x", 1: "y", 2: "z"}.get(axis, axis)
+    iu, iv = _FRAME_AXES[ax]
+    size, pixels = float(size), int(pixels)
+    c = -size + (np.arange(pixels) + 0.5) * ((size - -size) / pixels)      # pixel centres, as sph_column_density places them
+    pts = np.empty((pixels * pixels, 3))
+    pts[:, "xyz".index(ax)] = float(offset)
+    pts[:, iu] = np.tile(c, pixels)
+    pts[:, iv] = np.repeat(c, pixels)
+    return engine.interpolate(pts, n_out=1)["rho"].reshape(pixels, pixels)
 
 
 def to_gray(img, log=True, decades=4.0):
@@ -54,6 +73,8 @@ def main(argv=None):
     ap.add_argument("--pixels", type=int, default=512)
     ap.add_argument("--out", default=None)
     ap.add_argument("--npy", default=None)
+    ap.add_argument("--slice", type=float, default=None, metavar="OFFSET",
+                    help="write the density on the plane axis = OFFSET instead of the column density")
     ap.add_argument("--device", type=int, default=0)
     a = ap.parse_args(argv)
     from .engine import Engine
@@ -64,12 +85,18 @@ def main(argv=None):
     b, s = read_data_from_file(a.save_file, p)
     with Engine(p, device=a.device) as e:
         e.upload(b, s)
-        img = column_density(e, a.axis, a.size, a.pixels)
+        if a.slice is None:
+            img = column_density(e, a.axis, a.size, a.pixels)
+        else:
+            img = density_slice(e, a.axis, a.slice, a.size, a.pixels)
     out = a.out or (a.save_file.rsplit(".", 1)[0] + ".pgm")
     save_pgm(out, img)
     if a.npy:
         np.save(a.npy, img)
-    print(f" wrote {out}: {a.pixels} x {a.pixels}, sum * pixel area = {img.sum() * (2 * a.size / a.pixels) ** 2!r} (mass in frame)")
+    if a.slice is None:
+        print(f" wrote {out}: {a.pixels} x {a.pixels}, sum * pixel area = {img.sum() * (2 * a.size / a.pixels) ** 2!r} (mass in frame)")
+    else:
+        print(f" wrote {out}: {a.pixels} x {a.pixels} density slice {a.axis} = {a.slice!r}, max {img.max()!r}")
 
 
 if __name__ == "__main__":

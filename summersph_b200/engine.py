@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SPH_B200_LIB") or os.path.join(_HERE, "libsph_b200.so")   # override: developer experiments only
 _LIB = None
 
+INTERP = ("rho", "vx", "vy", "vz", "u", "alpha", "count")      # the SPH_INTERP_COUNT output columns of sph_interpolate
 STAGES = ("keys", "sort", "tree", "density", "gravity", "sph", "integrate", "h_iter", "cull", "comm", "halo", "let", "migrate", "gravity_near")
 
 
@@ -78,6 +79,7 @@ def load_library(path=None):
     lib.sph_conserved.argtypes = [vp, vp, i32]
     lib.sph_download_sink_spin.argtypes = [vp, vp, vp, vp]
     lib.sph_column_density.argtypes = [vp, i32, dbl, dbl, dbl, dbl, i32, i32, vp]
+    lib.sph_interpolate.argtypes = [vp, i64, vp, vp, vp, vp, i32]
     if path is None:
         _LIB = lib
     return lib
@@ -313,6 +315,18 @@ class Engine:
         u0, u1, v0, v1 = (float(e) for e in extent)
         self._ck(self._l.sph_column_density(self._c, int(ax), u0, u1, v0, v1, nu, nv, _p(img)))
         return img
+
+    def interpolate(self, points, n_out=len(INTERP)):
+        """The SPH interpolant of the resident gas at the rows of `points` ((M, 3): x, y, z), computed on the device
+        (`sph_interpolate`): dict of length-M arrays {rho, vx, vy, vz, u, alpha, count} truncated to the first `n_out`.
+        rho = sum m_j W(|x - x_j|, h_j), the means are mass-weighted (sum m_j f_j W / rho, 0 where rho = 0), count = the
+        number of particles with |x - x_j| <= 2 h_j.  Collective under the Morton domains: every rank passes the same points."""
+        pts = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+        m = len(pts)
+        cols = [np.ascontiguousarray(pts[:, k]) for k in range(3)]
+        out = np.zeros(max(int(n_out), 0) * m)
+        self._ck(self._l.sph_interpolate(self._c, m, *[_p(c) for c in cols], _p(out), int(n_out)))
+        return {k: out[i * m:(i + 1) * m] for i, k in enumerate(INTERP[:n_out])}
 
     def group_count(self):
         return int(self._l.sph_group_count(self._c))
