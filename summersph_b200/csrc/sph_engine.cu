@@ -60,7 +60,7 @@ struct sph_ctx {
   sph_params p; DevParams dp; int device = 0; int n_sm = 148; int max_smem = 0; cudaStream_t stream = nullptr;
   std::string err;
   int64_t n = 0, cap = 0, n_upload = 0; int n_sink = 0;
-  // particle state, double buffered for the Morton re-order / compaction
+  // particle state, double buffered for the Morton re-order / compaction; between calls the spare buffer is scratch (sph_download_neighbours)
   double* st[2][10] = {}; int* id[2] = {}; int cur = 0;
   double *rho = nullptr, *omega = nullptr, *prs = nullptr, *cs = nullptr, *por2 = nullptr;
   double *ax = nullptr, *ay = nullptr, *az = nullptr, *udot = nullptr, *adot = nullptr;
@@ -490,6 +490,24 @@ int flush_late(sph_ctx* c, unsigned need) {
   return SPH_OK;
 }
 enum { LF_H = 1u << 9, LF_M = 1u << 7, LF_U = 1u << 6, LF_ALL = 0x3ffu };
+
+// ascending-number position of every listed particle: the rank of its id among the ids present (all on device)
+__global__ void k_mark_present(int n, const int* __restrict__ id, int* __restrict__ present) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) present[id[i]] = 1;
+}
+__global__ void k_rank_of(int n, const int* __restrict__ id, const int* __restrict__ rank, int* __restrict__ pos) {
+  int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) pos[i] = rank[id[i]];
+}
+// pos[i] = rank of id[i] among id[0 .. n); cnt / off: n_upload + 1 ints of scratch, off keeps the rank of every id
+int id_ranks(sph_ctx* c, int n, const int* id, int* cnt, int* off, int* pos) {
+  const int nu = (int)c->n_upload, T = 256;
+  CK(cudaMemsetAsync(cnt, 0, sizeof(int) * (size_t)(nu + 1), c->stream));
+  LAUNCH(k_mark_present, cdiv(n, T), T, 0, n, id, cnt);
+  size_t bytes = c->cub_bytes;
+  CK(cub::DeviceScan::ExclusiveSum(c->cub_tmp, bytes, cnt, off, nu + 1, c->stream));
+  LAUNCH(k_rank_of, cdiv(n, T), T, 0, n, id, off, pos);
+  return SPH_OK;
+}
 
 #include "sph_domain_host.inl"
 
@@ -940,7 +958,7 @@ int io_fetch(sph_ctx* c, const int* fields, int nf) {
   for (int k = 0; k < nf && used < 5; ++k) {
     const int f = fields[k];
     if (!c->io_out[f]) continue;
-    LAUNCH(k_scatter_d, cdiv(n, T), T, 0, n, c->id[c->cur], c->st[c->cur][f], c->io_stage[used]);
+    LAUNCH(k_scatter<double>, cdiv(n, T), T, 0, n, c->id[c->cur], c->st[c->cur][f], c->io_stage[used]);
     fl[used++] = f;
   }
   if (!used) return SPH_OK;
@@ -1056,36 +1074,36 @@ int step(sph_ctx* c) {
   return SPH_OK;
 }
 
-// ascending-number position of every sorted particle: rank of its id among the surviving ids (all on device)
-__global__ void k_mark_present(int n, const int* __restrict__ id, int* __restrict__ present) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) present[id[i]] = 1;
-}
-__global__ void k_rank_of(int n, const int* __restrict__ id, const int* __restrict__ rank, int* __restrict__ pos) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) pos[i] = rank[id[i]];
-}
-int compute_pos(sph_ctx* c) {
-  const int n = (int)c->n, T = 256;
-  if ((int64_t)n == c->n_upload) {         // nothing was ever removed: number == upload index
-    CK(cudaMemcpyAsync(c->pos, c->id[c->cur], (size_t)n * 4, cudaMemcpyDeviceToDevice, c->stream));
+// ---- host-facing downloads: the rows in ascending-number order (sph_download, _diag, _tree, _neighbours, sph_step_host)
+// Rows covered: under domains every rank's own rows, otherwise this rank's (all of them in the replicated form).
+int64_t download_count(const sph_ctx* c) { return c->dd ? c->n_global : c->n; }
+// The ascending-number position of every covered row: dd_gpos under domains (collective), else pos.
+int download_rows(sph_ctx* c) {
+  if (c->dd) return dd_prepare_download(c);
+  if (c->n == c->n_upload) {         // nothing was ever removed: number == upload index
+    CK(cudaMemcpyAsync(c->pos, c->id[c->cur], (size_t)c->n * 4, cudaMemcpyDeviceToDevice, c->stream));
     return SPH_OK;
   }
-  const int nu = (int)c->n_upload;          // <= cap: cnt/off (cap + 1 ints) are only read while the octree is being built
-  CK(cudaMemsetAsync(c->cnt, 0, sizeof(int) * (size_t)(nu + 1), c->stream));
-  LAUNCH(k_mark_present, cdiv(n, T), T, 0, n, c->id[c->cur], c->cnt);
-  size_t bytes = c->cub_bytes;
-  CK(cub::DeviceScan::ExclusiveSum(c->cub_tmp, bytes, c->cnt, c->off, nu + 1, c->stream));
-  LAUNCH(k_rank_of, cdiv(n, T), T, 0, n, c->id[c->cur], c->off, c->pos);
-  return SPH_OK;
+  return id_ranks(c, (int)c->n, c->id[c->cur], c->cnt, c->off, c->pos);      // n_upload <= cap: cnt / off (cap + 1 ints) are only read while the octree is being built
 }
-// scatter into ascending-number order on the device, then one D2H per field; two staging buffers let the
-// scatter of field f+1 overlap nothing it depends on (stream order protects the buffers), one sync at the end
-int fetch_ordered(sph_ctx* c, const double* src, double* dst_host) {
+// One column of the covered rows to the host in ascending-number order (elem = 4 or 8 bytes; nothing if dst_host is null).
+// Domains: the ranks' own values are gathered in rank order into the first half of dd_gstage, then scattered into the
+// second.  Otherwise the scatter reads the column in place and alternates between two staging buffers, so the scatter of
+// the next column overlaps nothing it depends on (stream order protects the buffers); the caller synchronises once.
+int fetch_column(sph_ctx* c, Column col, size_t elem, void* dst_host) {
   if (!dst_host) return SPH_OK;
-  const int n = (int)c->n, T = 256;
-  double* stage = c->stage_flip ? c->stage_d2 : c->stage_d;
-  c->stage_flip ^= 1;
-  LAUNCH(k_scatter_d, cdiv(n, T), T, 0, n, c->pos, src, stage);
-  CK(cudaMemcpyAsync(dst_host, stage, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream));
+  const int n = (int)download_count(c), T = 256;
+  const void* src; void* stage; const int* pos;
+  if (c->dd) {
+    { int r_ = dd_gather(c, col, elem, c->dd_gstage); if (r_) return r_; }
+    src = c->dd_gstage; stage = c->dd_gstage + c->dd_g_cap; pos = c->dd_gpos;
+  } else {
+    src = dd_exported(c)[column_slot(col, c->cur, c->key[0] == c->key_alloc[0] ? 0 : 1)];
+    stage = c->stage_flip ? c->stage_d2 : c->stage_d; c->stage_flip ^= 1; pos = c->pos;
+  }
+  if (elem == 4) LAUNCH(k_scatter<int>, cdiv(n, T), T, 0, n, pos, (const int*)src, (int*)stage);
+  else LAUNCH(k_scatter<unsigned long long>, cdiv(n, T), T, 0, n, pos, (const unsigned long long*)src, (unsigned long long*)stage);
+  CK(cudaMemcpyAsync(dst_host, stage, (size_t)n * elem, cudaMemcpyDeviceToHost, c->stream));
   return SPH_OK;
 }
 int fetch_sink(sph_ctx* c, const double* src, double* dst_host) {
@@ -1627,8 +1645,8 @@ int sph_step_host(sph_ctx* c, int64_t n, const double* const* gas_in, int32_t ns
   if (gas_out && c->n > 0) {
     unsigned have = c->io_fetched;
     if (c->n != c->n_upload) { CK(cudaStreamSynchronize(c->io_stream)); have = 0; }      // rows were removed after the early columns left: all of them again, compacted
-    if ((r = compute_pos(c))) return r;
-    for (int f = 0; f < 10; ++f) if (!((have >> f) & 1u)) { if ((r = fetch_ordered(c, c->st[c->cur][f], gas_out[f]))) return r; }
+    if ((r = download_rows(c))) return r;
+    for (int f = 0; f < 10; ++f) if (!((have >> f) & 1u)) { if ((r = fetch_column(c, {DS_ST + f, CB_STATE}, 8, gas_out[f]))) return r; }
   }
   if (sink_out) {
     const double* ss[8] = {c->S.x, c->S.y, c->S.z, c->S.vx, c->S.vy, c->S.vz, c->S.m, c->S.radius};
@@ -1681,15 +1699,10 @@ int sph_download(sph_ctx* c, double* x, double* y, double* z, double* vx, double
   cudaSetDevice(c->device);
   int r;
   const bool any_gas = x || y || z || vx || vy || vz || u || m || alpha || h;
-  if (!any_gas) {}
-  else if (c->dd) {      // every rank receives all rows (tests, saves of small runs); production hosts use sph_download_local
-    if ((r = dd_prepare_download(c))) return r;
+  if (any_gas && download_count(c) > 0) {      // under domains every rank receives all rows (tests, saves of small runs); production hosts use sph_download_local
+    if ((r = download_rows(c))) return r;
     double* dst[10] = {x, y, z, vx, vy, vz, u, m, alpha, h};
-    for (int f = 0; f < 10; ++f) if ((r = dd_fetch_ordered(c, DS_ST + f, 3, dst[f]))) return r;
-  } else if (c->n > 0) {
-    if ((r = compute_pos(c))) return r;
-    double* dst[10] = {x, y, z, vx, vy, vz, u, m, alpha, h};
-    for (int f = 0; f < 10; ++f) if ((r = fetch_ordered(c, c->st[c->cur][f], dst[f]))) return r;
+    for (int f = 0; f < 10; ++f) if ((r = fetch_column(c, {DS_ST + f, CB_STATE}, 8, dst[f]))) return r;
   }
   double* sd[8] = {sx, sy, sz, svx, svy, svz, sm, srad};
   const double* ss[8] = {c->S.x, c->S.y, c->S.z, c->S.vx, c->S.vy, c->S.vz, c->S.m, c->S.radius};
@@ -1754,26 +1767,15 @@ int sph_download_diag(sph_ctx* c, double* rho, double* omega, double* pressure, 
                       double* ax, double* ay, double* az, double* udot, double* alphadot,
                       double* sax, double* say, double* saz) {
   if (!c) return SPH_ERR_ARG;
-  if (c->n <= 0) { c->err = "no particles"; return SPH_ERR_STATE; }
+  if (download_count(c) <= 0) { c->err = "no particles"; return SPH_ERR_STATE; }
   cudaSetDevice(c->device);
   int r;
-  if (c->dd) {
-    if ((r = dd_prepare_download(c))) return r;
-    const int slots[9] = {DS_RHO, DS_OMEGA, DS_PRS, DS_CS, DS_AX, DS_AY, DS_AZ, DS_UDOT, DS_ADOT};
-    double* dst[9] = {rho, omega, pressure, sound, ax, ay, az, udot, alphadot};
-    for (int f = 0; f < 9; ++f) if ((r = dd_fetch_ordered(c, slots[f], 0, dst[f]))) return r;
-    if ((r = fetch_sink(c, c->S.ax, sax))) return r;
-    if ((r = fetch_sink(c, c->S.ay, say))) return r;
-    if ((r = fetch_sink(c, c->S.az, saz))) return r;
-    CK(cudaStreamSynchronize(c->stream));
-    return SPH_OK;
-  }
-  if ((r = compute_pos(c))) return r;
-  // Omega and P stay rank-local during a step, and calc_smoothing rewrites rho / Omega of the particles it iterated (V:535): bring every slice up to date
-  { double* bufs[3] = {c->omega, c->prs, c->rho}; if ((r = allgatherv(c, bufs, 3))) return r; }
-  const double* src[9] = {c->rho, c->omega, c->prs, c->cs, c->ax, c->ay, c->az, c->udot, c->adot};
+  if ((r = download_rows(c))) return r;
+  // replicated: Omega and P stay rank-local during a step, and calc_smoothing rewrites rho / Omega of the particles it iterated (V:535): bring every slice up to date
+  if (!c->dd) { double* bufs[3] = {c->omega, c->prs, c->rho}; if ((r = allgatherv(c, bufs, 3))) return r; }
+  const int slots[9] = {DS_RHO, DS_OMEGA, DS_PRS, DS_CS, DS_AX, DS_AY, DS_AZ, DS_UDOT, DS_ADOT};
   double* dst[9] = {rho, omega, pressure, sound, ax, ay, az, udot, alphadot};
-  for (int f = 0; f < 9; ++f) if ((r = fetch_ordered(c, src[f], dst[f]))) return r;
+  for (int f = 0; f < 9; ++f) if ((r = fetch_column(c, {slots[f], CB_FIXED}, 8, dst[f]))) return r;
   if ((r = fetch_sink(c, c->S.ax, sax))) return r;
   if ((r = fetch_sink(c, c->S.ay, say))) return r;
   if ((r = fetch_sink(c, c->S.az, saz))) return r;
@@ -1787,48 +1789,18 @@ int sph_download_tree(sph_ctx* c, int32_t* order, uint64_t* key, int32_t* level,
   if (!c->tree_valid) { c->err = "no tree"; return SPH_ERR_STATE; }
   cudaSetDevice(c->device);
   int r;
-  if (c->dd) {      // the global depth-first order = the domains' orders in rank order
-    if ((r = dd_prepare_download(c))) return r;
-    const int n = (int)c->n_global, T = 256;
-    if (order) { CK(cudaMemcpyAsync(order, c->dd_gpos, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream)); }
-    if (key) {
-      if ((r = dd_gather(c, DS_KEY, 2, 8, c->dd_gstage))) return r;
-      LAUNCH(k_scatter_u64, cdiv(n, T), T, 0, n, c->dd_gpos, (const unsigned long long*)c->dd_gstage, (unsigned long long*)(c->dd_gstage + c->dd_g_cap));
-      CK(cudaMemcpyAsync(key, c->dd_gstage + c->dd_g_cap, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-    }
-    std::vector<int> lev(n);
-    if (level || size) {
-      if ((r = dd_gather(c, DS_LEVEL, 0, 4, c->dd_gstage))) return r;
-      LAUNCH(k_scatter_i, cdiv(n, T), T, 0, n, c->dd_gpos, (const int*)c->dd_gstage, (int*)(c->dd_gstage + c->dd_g_cap));
-      CK(cudaMemcpyAsync(lev.data(), c->dd_gstage + c->dd_g_cap, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-      if (level) std::memcpy(level, lev.data(), (size_t)n * 4);
-    }
-    if ((r = dd_fetch_ordered(c, DS_LCX, 0, cx))) return r;
-    if ((r = dd_fetch_ordered(c, DS_LCY, 0, cy))) return r;
-    if ((r = dd_fetch_ordered(c, DS_LCZ, 0, cz))) return r;
-    if (size) {
-      RootBox rb; CK(cudaMemcpy(&rb, c->root, sizeof(rb), cudaMemcpyDeviceToHost));
-      for (int i = 0; i < n; ++i) { double s = rb.size; for (int q = 0; q < lev[i]; ++q) s *= 0.5; size[i] = s; }
-    }
-    return SPH_OK;
-  }
-  const int n = (int)c->n, T = 256;
-  if ((r = compute_pos(c))) return r;
-  if (order) { CK(cudaMemcpyAsync(order, c->pos, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream)); }
-  if (key) {
-    LAUNCH(k_scatter_u64, cdiv(n, T), T, 0, n, c->pos, (const unsigned long long*)c->key[0], (unsigned long long*)c->stage_d);
-    CK(cudaMemcpyAsync(key, c->stage_d, (size_t)n * 8, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-  }
+  if ((r = download_rows(c))) return r;
+  const int n = (int)download_count(c);
+  // the global depth-first order = the positions of the rows (under domains: the domains' orders in rank order)
+  if (order) CK(cudaMemcpyAsync(order, c->dd ? c->dd_gpos : c->pos, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
   std::vector<int> lev(n);
-  if (level || size) {
-    LAUNCH(k_scatter_i, cdiv(n, T), T, 0, n, c->pos, c->level, (int*)c->stage_d);
-    CK(cudaMemcpyAsync(lev.data(), c->stage_d, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-    if (level) std::memcpy(level, lev.data(), (size_t)n * 4);
-  }
-  if ((r = fetch_ordered(c, c->lcx, cx))) return r;
-  if ((r = fetch_ordered(c, c->lcy, cy))) return r;
-  if ((r = fetch_ordered(c, c->lcz, cz))) return r;
+  if ((r = fetch_column(c, {DS_KEY, CB_KEY}, 8, key))) return r;
+  if ((r = fetch_column(c, {DS_LEVEL, CB_FIXED}, 4, level || size ? lev.data() : nullptr))) return r;
+  if ((r = fetch_column(c, {DS_LCX, CB_FIXED}, 8, cx))) return r;
+  if ((r = fetch_column(c, {DS_LCY, CB_FIXED}, 8, cy))) return r;
+  if ((r = fetch_column(c, {DS_LCZ, CB_FIXED}, 8, cz))) return r;
   CK(cudaStreamSynchronize(c->stream));
+  if (level) std::memcpy(level, lev.data(), (size_t)n * 4);
   if (size) {
     RootBox rb; CK(cudaMemcpy(&rb, c->root, sizeof(rb), cudaMemcpyDeviceToHost));
     for (int i = 0; i < n; ++i) { double s = rb.size; for (int q = 0; q < lev[i]; ++q) s *= 0.5; size[i] = s; }
@@ -1839,60 +1811,41 @@ int sph_download_tree(sph_ctx* c, int32_t* order, uint64_t* key, int32_t* level,
 int sph_download_neighbours(sph_ctx* c, int32_t* count, uint64_t* hash, int64_t* offsets, int32_t* list, int64_t list_cap) {
   if (!c) return SPH_ERR_ARG;
   if (!c->tree_valid) { c->err = "no tree"; return SPH_ERR_STATE; }
+  if (c->dd && list) { c->err = "sph_download_neighbours: the list form is not available under the domain decomposition"; return SPH_ERR_STATE; }
   cudaSetDevice(c->device);
-  const int n = (int)c->n, W = 8;
   int r;
-  if (c->dd) {      // counts and hashes of all ranks' own particles (the CSR list form is single-rank / replicated only)
-    if (list) { c->err = "sph_download_neighbours: the list form is not available under the domain decomposition"; return SPH_ERR_STATE; }
-    if ((r = dd_prepare_download(c))) return r;
-    const int ng = (int)c->n_global, T = 256;
-    size_t smem = (size_t)W * 4 * WALK_TILE * 8 + (size_t)W * WALK_TILE * 4 + (size_t)W * WALK_WS * 4;
-    LAUNCH(k_neighbours, walk_grid(c, W), W * 32, smem, c->g1, c->groups, dens_arrays(c), c->pos, c->bvh, c->bi, (int*)c->stage_d, (unsigned long long*)c->stage_d2, nullptr, nullptr);
-    std::vector<int> cnt(ng); std::vector<unsigned long long> hs(ng);
-    if ((r = dd_gather(c, DS_STAGE1, 0, 4, c->dd_gstage))) return r;
-    LAUNCH(k_scatter_i, cdiv(ng, T), T, 0, ng, c->dd_gpos, (const int*)c->dd_gstage, (int*)(c->dd_gstage + c->dd_g_cap));
-    CK(cudaMemcpyAsync(cnt.data(), c->dd_gstage + c->dd_g_cap, (size_t)ng * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-    if ((r = dd_gather(c, DS_STAGE2, 0, 8, c->dd_gstage))) return r;
-    LAUNCH(k_scatter_u64, cdiv(ng, T), T, 0, ng, c->dd_gpos, (const unsigned long long*)c->dd_gstage, (unsigned long long*)(c->dd_gstage + c->dd_g_cap));
-    CK(cudaMemcpyAsync(hs.data(), c->dd_gstage + c->dd_g_cap, (size_t)ng * 8, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-    if (count) std::memcpy(count, cnt.data(), (size_t)ng * 4);
-    if (hash) std::memcpy(hash, hs.data(), (size_t)ng * 8);
-    if (offsets) { offsets[0] = 0; for (int i = 0; i < ng; ++i) offsets[i + 1] = offsets[i] + cnt[i]; }
-    return SPH_OK;
-  }
-  if ((r = compute_pos(c))) return r;
-  int* d_count = nullptr; unsigned long long* d_hash = nullptr; long long* d_off = nullptr; int* d_list = nullptr;
-  DA(d_count, n); DA(d_hash, n);
-  size_t smem = (size_t)W * 4 * WALK_TILE * 8 + (size_t)W * WALK_TILE * 4 + (size_t)W * WALK_WS * 4;
-  LAUNCH(k_neighbours, walk_grid(c, W), W * 32, smem, c->n_groups, c->groups, dens_arrays(c), c->pos, c->bvh, c->bi, d_count, d_hash, nullptr, nullptr);
-  std::vector<int> cnt_sorted(n), pos(n), cnt_num(n);
-  std::vector<unsigned long long> hash_sorted(n);
+  if ((r = download_rows(c))) return r;
+  const int n = (int)download_count(c), W = 8, own_groups = c->n_groups - c->ng_halo;
+  const size_t smem = (size_t)W * 4 * WALK_TILE * 8 + (size_t)W * WALK_TILE * 4 + (size_t)W * WALK_WS * 4;
+  // counts and hashes of the own rows (the walk groups but the halo's), in sorted order, land in the state buffers that
+  // are not current: nothing reads those between calls (the next re-order or upload overwrites them), and the staging
+  // buffers stay free for the scatter
+  const StateArrays spare = state_of(c, c->cur ^ 1);
+  int* const d_count = (int*)spare.x; unsigned long long* const d_hash = (unsigned long long*)spare.y;
+  LAUNCH(k_neighbours, walk_grid(c, W), W * 32, smem, own_groups, c->groups, dens_arrays(c), c->pos, c->bvh, c->bi, d_count, d_hash, nullptr, nullptr);
+  std::vector<int> cnt(n);
+  if ((r = fetch_column(c, {DS_ST + 0, CB_SPARE_STATE}, 4, cnt.data()))) return r;
+  if ((r = fetch_column(c, {DS_ST + 1, CB_SPARE_STATE}, 8, hash))) return r;
   CK(cudaStreamSynchronize(c->stream));
-  CK(cudaMemcpy(cnt_sorted.data(), d_count, (size_t)n * 4, cudaMemcpyDeviceToHost));
-  CK(cudaMemcpy(hash_sorted.data(), d_hash, (size_t)n * 8, cudaMemcpyDeviceToHost));
+  if (count) std::memcpy(count, cnt.data(), (size_t)n * 4);
+  std::vector<long long> off(n + 1, 0);
+  for (int i = 0; i < n; ++i) off[i + 1] = off[i] + cnt[i];
+  if (offsets) std::memcpy(offsets, off.data(), (size_t)(n + 1) * 8);
+  if (!list) return SPH_OK;
+  const long long tot = off[n];
+  if (tot > list_cap) { c->err = "neighbour list capacity too small: need " + std::to_string(tot) + " have " + std::to_string((long long)list_cap); return SPH_ERR_ARG; }
+  // the list form (single rank / replicated): every row's list is written at its offset, so the offsets go in sorted order
+  std::vector<int> pos(n); std::vector<long long> off_sorted(n);
   CK(cudaMemcpy(pos.data(), c->pos, (size_t)n * 4, cudaMemcpyDeviceToHost));
-  for (int i = 0; i < n; ++i) { cnt_num[pos[i]] = cnt_sorted[i]; if (hash) hash[pos[i]] = hash_sorted[i]; }
-  if (count) std::memcpy(count, cnt_num.data(), (size_t)n * 4);
-  std::vector<long long> off_num(n + 1, 0);
-  for (int i = 0; i < n; ++i) off_num[i + 1] = off_num[i] + cnt_num[i];
-  if (offsets) for (int i = 0; i <= n; ++i) offsets[i] = off_num[i];
-  int rc = SPH_OK;
-  if (list) {
-    const long long tot = off_num[n];
-    if (tot > list_cap) { c->err = "neighbour list capacity too small: need " + std::to_string(tot) + " have " + std::to_string((long long)list_cap); rc = SPH_ERR_ARG; }
-    else {
-      std::vector<long long> off_sorted(n);
-      for (int i = 0; i < n; ++i) off_sorted[i] = off_num[pos[i]];
-      DA(d_off, n); DA(d_list, std::max<long long>(tot, 1));
-      CK(cudaMemcpyAsync(d_off, off_sorted.data(), (size_t)n * 8, cudaMemcpyHostToDevice, c->stream));
-      LAUNCH(k_neighbours, walk_grid(c, W), W * 32, smem, c->n_groups, c->groups, dens_arrays(c), c->pos, c->bvh, c->bi, d_count, d_hash, d_off, d_list);
-      CK(cudaMemcpyAsync(list, d_list, (size_t)tot * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
-      for (int i = 0; i < n; ++i) std::sort(list + off_num[i], list + off_num[i + 1]);
-    }
-  }
-  CK(cudaStreamSynchronize(c->stream));
-  cudaFree(d_count); cudaFree(d_hash); if (d_off) cudaFree(d_off); if (d_list) cudaFree(d_list);
-  return rc;
+  for (int i = 0; i < n; ++i) off_sorted[i] = off[pos[i]];
+  long long* const d_off = (long long*)spare.z; int* d_list = nullptr;
+  DA(d_list, std::max<long long>(tot, 1));
+  CK(cudaMemcpyAsync(d_off, off_sorted.data(), (size_t)n * 8, cudaMemcpyHostToDevice, c->stream));
+  LAUNCH(k_neighbours, walk_grid(c, W), W * 32, smem, own_groups, c->groups, dens_arrays(c), c->pos, c->bvh, c->bi, d_count, d_hash, d_off, d_list);
+  CK(cudaMemcpyAsync(list, d_list, (size_t)tot * 4, cudaMemcpyDeviceToHost, c->stream)); CK(cudaStreamSynchronize(c->stream));
+  cudaFree(d_list);
+  for (int i = 0; i < n; ++i) std::sort(list + off[i], list + off[i + 1]);
+  return SPH_OK;
 }
 
 int sph_set_exact_counters(sph_ctx* c, int32_t on) {

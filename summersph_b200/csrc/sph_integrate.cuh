@@ -301,13 +301,7 @@ __global__ void k_iota(int n, int* a) { int i = blockIdx.x * blockDim.x + thread
 // scatter by id for downloads in ascending number order: out[rank(id)] ; ids are persistent upload indices,
 // so the ascending-number position of a particle is its rank among surviving ids (computed on the host side
 // from the id array, see sph_engine.cu).
-__global__ void k_scatter_d(int n, const int* __restrict__ pos, const double* __restrict__ src, double* __restrict__ dst) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) dst[pos[i]] = src[i];
-}
-__global__ void k_scatter_i(int n, const int* __restrict__ pos, const int* __restrict__ src, int* __restrict__ dst) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) dst[pos[i]] = src[i];
-}
-__global__ void k_scatter_u64(int n, const int* __restrict__ pos, const unsigned long long* __restrict__ src, unsigned long long* __restrict__ dst) {
+template <class T> __global__ void k_scatter(int n, const int* __restrict__ pos, const T* __restrict__ src, T* __restrict__ dst) {
   int i = blockIdx.x * blockDim.x + threadIdx.x; if (i < n) dst[pos[i]] = src[i];
 }
 

@@ -31,7 +31,7 @@ def main():
     token = sys.argv[8] if len(sys.argv) > 8 else ""
     n = int(sys.argv[9]) if len(sys.argv) > 9 else 60_000
     domains = int(sys.argv[10]) if len(sys.argv) > 10 else 0
-    from summersph_b200.engine import Engine
+    from summersph_b200.engine import Engine, SphError
     from summersph_b200.state import GAS_FIELDS
     p, b, s = case(mode, n, domains)
     with Engine(p, device=device) as e:
@@ -42,6 +42,8 @@ def main():
                 e.comm_init_host(rank, world, token)
         if len(sys.argv) > 12 and sys.argv[12] == "devics":
             e.ics_disc(n, seed=12)           # every rank generates its own rows on the device
+        elif len(sys.argv) > 12 and sys.argv[12] == "rank0":
+            e.upload_local(n, b if rank == 0 else b.take(slice(0, 0)), s)      # domains: rank 0 owns every row, the others none
         else:
             e.upload(b, s)
         dt, t = 0.01, 0.0
@@ -65,6 +67,13 @@ def main():
             d2 = e.diag(); extra.update({"e_" + k: v for k, v in d2.items()})
             c2 = e.counters(); extra["e_counters"] = np.array([c2[k] for k in sorted(c2)], dtype=np.int64)
             extra["local_n"] = np.array([e.local_size()])
+        if len(sys.argv) > 11 and sys.argv[11] == "nblist":      # the neighbour list form after an evaluation: its error code, 0 if it worked
+            e.evaluate()
+            try:
+                e.neighbours(with_list=True)
+                extra["nblist_code"] = np.array([0])
+            except SphError as err:
+                extra["nblist_code"] = np.array([err.code]); extra["nblist_msg"] = np.array([str(err)])
         res = {k: getattr(bb, k) for k in GAS_FIELDS}
         res.update({"s_" + k: getattr(ss, k) for k in ("x", "y", "z", "vx", "vy", "vz", "m")})
         res.update({"d_" + k: v for k, v in d.items()})
