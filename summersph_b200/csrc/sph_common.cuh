@@ -19,6 +19,11 @@
 #define SPH_MAX_SINKS 64
 #define FULL_MASK 0xffffffffu
 
+#ifdef SCREEN_AUDIT    // developer build (scripts/build_variant.sh audit -DSCREEN_AUDIT): decisions of the FP32 screens that the FP64
+                       // tests they stand in front of contradict: [0] density, [1] pair loop, [2] gravity (stderr per evaluation / step)
+__device__ unsigned long long screen_audit[3];
+#endif
+
 struct DevParams {
   int    variable_h;     // V mode
   int    soft_hi;        // T:298 softening

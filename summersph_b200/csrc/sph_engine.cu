@@ -1573,6 +1573,13 @@ int sph_upload_local(sph_ctx* c, int64_t n_global, int64_t id_first, const int32
   return upload_impl(c, n_global, id_first, n_local, src, ns, ssrc, srad, false, 0, number);
 }
 
+#ifdef SCREEN_AUDIT
+static void screen_audit_report(sph_ctx* c, const char* what) {
+  unsigned long long d[3]; cudaStreamSynchronize(c->stream); cudaMemcpyFromSymbol(d, screen_audit, sizeof(d)); unsigned long long z[3] = {}; cudaMemcpyToSymbol(screen_audit, z, sizeof(z));
+  fprintf(stderr, "SCREEN_AUDIT %s density %llu pair %llu gravity %llu\n", what, d[0], d[1], d[2]);
+}
+#endif
+
 int sph_evaluate(sph_ctx* c, int32_t mask) {
   if (!c) return SPH_ERR_ARG;
   if (c->n <= 0) { c->err = "no particles uploaded"; return SPH_ERR_STATE; }
@@ -1582,6 +1589,9 @@ int sph_evaluate(sph_ctx* c, int32_t mask) {
   CK(cudaMemcpyAsync(c->h_sc, c->sc, sizeof(SimScalars), cudaMemcpyDeviceToHost, c->stream));
   if ((r = fetch_counters(c))) return r;
   c->far_n_ovf = c->h_sc->far_ovf;
+#ifdef SCREEN_AUDIT
+  screen_audit_report(c, "evaluate");
+#endif
   stage_collect(c, true);
   CK(cudaGetLastError());
   return check_device_error(c);
@@ -1596,6 +1606,9 @@ int sph_step(sph_ctx* c, double* dt, double* t, int64_t* n_out, int32_t* ns_out)
   int r = step(c); if (r) return r;
   if ((r = fetch_counters(c))) return r;
   c->counts.h_iterations = (int64_t)c->h_ctr->h_iters;
+#ifdef SCREEN_AUDIT
+  screen_audit_report(c, "step");
+#endif
   stage_collect(c, true);
   CK(cudaGetLastError());
   *dt = c->h_sc->dt; *t = c->h_sc->t;

@@ -52,6 +52,7 @@ struct GravWarpSmem {
   unsigned lmask[GW_LIST];
   double   mcx[32], mcy[32], mcz[32], msize[32], mlo[32], mhi[32];   // mixed nodes of the current trip: COM, size, d2 band of the cheap FP64 test
   float4   mf[32];                                                   // the same nodes for the FP32 screen: COM relative to the run's origin, size^2 / theta^2
+                                                                     //   (NaN: the screen cannot decide for this run, every particle takes the FP64 test)
   unsigned mmask[32];
   double   nacc[3][32];                                              // full walk: the near sums of the lanes between list evaluations (registers are short there)
   double   hpar[3][32];                                              // full walk: 1/h, 4 h^2, hc2 of the lanes (only the near entries need them)
@@ -151,6 +152,14 @@ __device__ __forceinline__ void sink_terms(const DevParams& P, const SinkArrays&
   }
 }
 
+#ifdef SCREEN_AUDIT
+// the reference's opening test, F:274-278, without contraction: accept the node
+__device__ __forceinline__ bool audit_mac_accept(double dx, double dy, double dz, double soft, double size, double theta) {
+  const double e2 = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)), soft);
+  return __ddiv_rn(size, __dsqrt_rn(e2)) < theta;
+}
+#endif
+
 // dynamic smem: grav table (nq+1 doubles, padded to even) then one GravWarpSmem per warp
 // MODE 0: full walk that stores the far sums and records the near pairs; MODE 1: near-only walk on top of the stored far
 // sums (see "Far-field reuse" above); MODE 2: full walk that stores nothing (no near / far split: one sum per particle)
@@ -242,8 +251,19 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
       const double soft_min = warp_min(live ? soft : INFINITY), soft_max = warp_max(live ? soft : 0.0);
       const unsigned livemask = __ballot_sync(FULL_MASK, live);
       // FP32 screens (classification against the run's box, and the per-particle test on mixed nodes): coordinates
-      // relative to the box centre, 3e-5 margins (float rounding of d^2 stays below ~1e-6 relative because
-      // d^2 >= soft); whatever falls inside a margin is decided by the FP64 tests below, so no decision changes.
+      // relative to the box centre g0.  A particle is within hw = max(hxf, hyf, hzf) of g0 per axis and a node's COM
+      // within rho = max |r| of it; each float coordinate carries 2^-24 of its magnitude and the float difference
+      // 2^-24 of at most hw + rho, so the float distance from a particle to a node is off by at most
+      // sqrt(3) 2^-23 (hw + rho) < delta = 4e-7 (hw + rho), and each per-axis distance by less than delta (the code
+      // takes the sums of the three half-widths and of the three |r| components, which bound hw and rho).  The run
+      // can be far wider than the distances decided on (runs straddle coarse cells), so delta is an absolute band:
+      // the classification shrinks the per-axis distances to the box by delta and grows the far ones by delta (3e-5
+      // relative margins on top for the float arithmetic).  A mixed node's per-particle test keeps its 3e-5 margins
+      // on W = size^2 / theta^2 where delta <= 1e-5 sqrt(W): the float distance d_f is within delta of d, so
+      // d_f^2 + soft moves by less than (1 +- 1e-5)^2 - 1 ~ 2e-5 of W around the decision, the margins' remaining 1e-5
+      // covers the float arithmetic of d^2 and W.  Where delta is larger the node's W is stored as NaN: both float
+      // comparisons fail and every particle takes the FP64 test.  Whatever falls inside a margin is decided by the
+      // FP64 tests below, so no decision changes.
       const double g0x = 0.5 * (lo0 + hi0), g0y = 0.5 * (lo1 + hi1), g0z = 0.5 * (lo2 + hi2);
       const float hxf = __double2float_ru(0.5 * (hi0 - lo0)) * 1.00001f, hyf = __double2float_ru(0.5 * (hi1 - lo1)) * 1.00001f, hzf = __double2float_ru(0.5 * (hi2 - lo2)) * 1.00001f;
       const float xif = (float)(xi - g0x), yif = (float)(yi - g0y), zif = (float)(zi - g0z);
@@ -279,7 +299,7 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
         // ---- lane = node: classify against the group box
         int cls = 0;                           // 1 all accept, 2 all open, 3 mixed
         double ncx = 0.0, ncy = 0.0, ncz = 0.0, nm = 0.0, nsize = 0.0; int nchild = 0, nnch = 0;
-        float rxf = 0.f, ryf = 0.f, rzf = 0.f, s2f = 0.f, dmin2 = 0.f;
+        float rxf = 0.f, ryf = 0.f, rzf = 0.f, s2f = 0.f, dmin2 = 0.f, dlt = 0.f;
         if (valid) {
           const double2* p = reinterpret_cast<const double2*>(wn + e.x);
           const double2 a = __ldg(p), b = __ldg(p + 1), c = __ldg(p + 2);
@@ -287,8 +307,9 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
           nchild = __double2loint(c.y); nnch = __double2hiint(c.y);
           rxf = (float)(ncx - g0x); ryf = (float)(ncy - g0y); rzf = (float)(ncz - g0z);
           const float axf = fabsf(rxf), ayf = fabsf(ryf), azf = fabsf(rzf);
-          const float nx = fmaxf(axf - hxf, 0.f), ny = fmaxf(ayf - hyf, 0.f), nz = fmaxf(azf - hzf, 0.f);
-          const float fx = axf + hxf, fy = ayf + hyf, fz = azf + hzf;
+          dlt = 4e-7f * ((hxf + hyf + hzf) + (axf + ayf + azf));
+          const float nx = fmaxf(axf - hxf - dlt, 0.f), ny = fmaxf(ayf - hyf - dlt, 0.f), nz = fmaxf(azf - hzf - dlt, 0.f);
+          const float fx = axf + hxf + dlt, fy = ayf + hyf + dlt, fz = azf + hzf + dlt;
           dmin2 = fmaf(nx, nx, fmaf(ny, ny, fmaf(nz, nz, softf_min)));
           const float dmax2 = fmaf(fx, fx, fmaf(fy, fy, fmaf(fz, fz, softf_max)));
           const float szf = (float)nsize;
@@ -303,6 +324,19 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
           }
         }
         const unsigned emask = (unsigned)e.y;
+#ifdef SCREEN_AUDIT
+        {   // the nodes classified for the whole run: the exact test of every particle of the node's lane set
+          unsigned bc = __ballot_sync(FULL_MASK, (cls == 1 || cls == 2) && nnch != 0), bad = 0;
+          while (bc) {
+            const int L = __ffs(bc) - 1; bc &= bc - 1;
+            const double cx = __shfl_sync(FULL_MASK, ncx, L), cy = __shfl_sync(FULL_MASK, ncy, L), cz = __shfl_sync(FULL_MASK, ncz, L), sz = __shfl_sync(FULL_MASK, nsize, L);
+            const int cl = __shfl_sync(FULL_MASK, cls, L);
+            const unsigned em = __shfl_sync(FULL_MASK, emask, L);
+            if ((em >> lane) & 1u) bad += audit_mac_accept(xi - cx, yi - cy, zi - cz, soft, sz, theta) != (cl == 1) ? 1u : 0u;
+          }
+          if (bad) atomicAdd(&screen_audit[2], (unsigned long long)bad);
+        }
+#endif
         const unsigned balM = __ballot_sync(FULL_MASK, cls == 3);
         const int nmix = __popc(balM);
         GWS(1, npop); GWS(2, __popc(__ballot_sync(FULL_MASK, valid && cls == 0))); GWS(3, __popc(__ballot_sync(FULL_MASK, cls == 1)));
@@ -313,7 +347,8 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
           // size^2 < theta^2 d2 (1 - 1e-12)  <=>  d2 > size^2 / (theta^2 (1 - 1e-12)); the band in between gets the exact test
           const double s2t = nsize * nsize * inv_theta2;
           W.mhi[pos] = s2t * (1.0 + 2e-12); W.mlo[pos] = s2t * (1.0 - 2e-12);
-          W.mf[pos] = make_float4(rxf, ryf, rzf, s2f * inv_th2f);
+          const float wf = s2f * inv_th2f;
+          W.mf[pos] = make_float4(rxf, ryf, rzf, dlt * dlt <= 1e-10f * wf ? wf : __int_as_float(0x7fffffff));
         }
         __syncwarp();
         // ---- lane = particle: the reference's own test on the mixed nodes; the node's lane keeps the two ballots
@@ -328,6 +363,10 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
           const float dxf = xif - mq.x, dyf = yif - mq.y, dzf = zif - mq.z;
           const float d2f = fmaf(dxf, dxf, fmaf(dyf, dyf, fmaf(dzf, dzf, softf)));
           bool accept = d2f > mq.w * (1.f + 3e-5f);
+#ifdef SCREEN_AUDIT
+          if (in && (accept || d2f < mq.w * (1.f - 3e-5f)) && audit_mac_accept(xi - W.mcx[q], yi - W.mcy[q], zi - W.mcz[q], soft, W.msize[q], theta) != accept)
+            atomicAdd(&screen_audit[2], 1ull);
+#endif
           if (!accept && !(d2f < mq.w * (1.f - 3e-5f))) {       // inside the float margin: the FP64 test
             const double dx = xi - W.mcx[q], dy = yi - W.mcy[q], dz = zi - W.mcz[q];          // F:274
             const double d2 = fma(dx, dx, fma(dy, dy, fma(dz, dz, soft)));
@@ -352,6 +391,19 @@ k_gravity(int g_begin, int g_end, const int2* __restrict__ groups, const BvhBox*
           W.lxy[pos] = make_double2(ncx, ncy); W.lzg[pos] = make_double2(ncz, P.G * nm); W.lmask[pos] = acc_mask;
           if (SPLIT) W.lidx[pos] = e.x;
         }
+#ifdef SCREEN_AUDIT
+        {   // far entries: no particle they are accepted for may lie within its near / far split
+          unsigned bf = balL, bad = 0;
+          while (bf) {
+            const int L = __ffs(bf) - 1; bf &= bf - 1;
+            const double cx = __shfl_sync(FULL_MASK, ncx, L), cy = __shfl_sync(FULL_MASK, ncy, L), cz = __shfl_sync(FULL_MASK, ncz, L);
+            const unsigned am = __shfl_sync(FULL_MASK, acc_mask, L);
+            const double dx = xi - cx, dy = yi - cy, dz = zi - cz;
+            if ((am >> lane) & 1u) bad += fma(dx, dx, fma(dy, dy, fma(dz, dz, soft))) <= hc2 ? 1u : 0u;
+          }
+          if (bad) atomicAdd(&screen_audit[2], (unsigned long long)bad);
+        }
+#endif
         nn += __popc(balN);
         ln += __popc(balL);
         GWS(6, __popc(balL)); GWS(7, __popc(balN));

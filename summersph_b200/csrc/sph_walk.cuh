@@ -317,10 +317,10 @@ struct DensityOp {
   }
   __device__ __forceinline__ void list_end() { __syncwarp(); list_flush(ln, true); __syncwarp(); }
   __device__ __forceinline__ void consume(int count) {
-    // Prefilter, lane = target, FP32 on group-relative coordinates: |x_i - x_j|^2 against 4 h_i^2 with a 1e-4 margin
-    // (float rounding is ~1e-6 of the limit).  Beyond it W(q > 2) = 0 exactly (F:112), so it only drops exact zeros;
-    // the reference's leaf-box test (F:443 | V:479) and q <= 2 are evaluated in FP64 on the survivors.  With the
-    // exact candidate counter on, every staged source goes through the FP64 tests.
+    // Prefilter, lane = target, FP32 on group-relative coordinates: |x_i - x_j|^2 against r2maxif, the square of
+    // b_i = 2 h_i + 4e-7 (gd + 2 h_i) (density_bound).  Beyond it W(q > 2) = 0 exactly (F:112), so it only drops
+    // exact zeros; the reference's leaf-box test (F:443 | V:479) and q <= 2 are evaluated in FP64 on the survivors.
+    // With the exact candidate counter on, every staged source goes through the FP64 tests.
     unsigned mask = 0;
     if (active) {
       if (count_all) mask = count >= 32 ? 0xffffffffu : ((1u << count) - 1u);
@@ -334,6 +334,21 @@ struct DensityOp {
         }
       }
     }
+#ifdef SCREEN_AUDIT
+    if (active && !count_all) {          // every staged source the screen dropped: would the FP64 test have summed it?
+      unsigned bad = 0;
+      for (int k = 0; k < count; ++k) {
+        if ((mask >> k) & 1u) continue;
+        const double R = sR[k], dx = xi - sx[k], dy = yi - sy[k], dz = zi - sz[k];
+        const bool box = (fabs(xi - scx[k]) < R) & (fabs(yi - scy[k]) < R) & (fabs(zi - scz[k]) < R);
+        const double r2 = dx * dx + dy * dy + dz * dz;
+        double r, rs; fast_sqrt_rsqrt(r2, r, rs);
+        r = (r2 == 0.0) ? 0.0 : r;
+        bad += (box & (r * inv_h <= 2.0)) ? 1u : 0u;
+      }
+      if (bad) atomicAdd(&screen_audit[0], (unsigned long long)bad);
+    }
+#endif
 #ifdef WALK_DEBUG
     { int hc = __popc(mask); int mx = hc, sm = hc; for (int o = 16; o > 0; o >>= 1) { mx = max(mx, __shfl_xor_sync(FULL_MASK, mx, o)); sm += __shfl_xor_sync(FULL_MASK, sm, o); }
       WKD(8, 1); WKD(9, count); WKD(10, mx); WKD(11, sm); }
@@ -366,6 +381,32 @@ struct DensityOp {
     contrib += in ? 1u : 0u;
   }
 };
+
+// Rounding bound of the walks' FP32 prefilters.  Coordinates are taken relative to g0, the centre of the group's
+// position box of half-width gd (largest axis).  A target is within gd of g0 per axis, and a source that can be a
+// member at distance r <= 2h within gd + 2h.  Each float coordinate carries at most 2^-24 of its magnitude and the float
+// difference 2^-24 of at most 2h: per axis the float difference is off by at most 2^-24 (2 gd + 4h), the float distance
+// by at most sqrt(3) 2^-24 (2 gd + 4h) < 4e-7 (gd + 2h).  So a member has r_float <= b = 2h + 4e-7 (gd + 2h); the fmaf
+// sum of squares adds < 1e-6 relative, which the caller's 1e-4 covers.  A fixed relative margin would not do: gd is
+// the group's width, unrelated to h (a sparse cell's bucket can be 1e4 h wide or more).
+__device__ __forceinline__ double group_half_width(const float* lo, const float* hi) {
+  return 0.5 * fmax(fmax((double)hi[0] - (double)lo[0], (double)hi[1] - (double)lo[1]), (double)hi[2] - (double)lo[2]);
+}
+__device__ __forceinline__ double walk_bound(double h, double gd) { return 2.0 * h + 4e-7 * (gd + 2.0 * h); }
+// The pair loop's limit for one side is r2max 1.00012 + pad, r2max = 4 h^2 (1 + 1e-9) (INFINITY: keep every partner),
+// rounded up: with c = 4e-7 gd, b^2 = (2h (1 + 4e-7) + c)^2 <= r2max (1 + 4e-7)^2 (1 + t) + c^2 (1 + 1/t) for any t > 0;
+// t = 1e-5 and the 1e-4 of the fmaf sum give r2max 1.00012 + 1.0001e5 c^2 (4.1e-7: the float arithmetic of c), and the
+// larger of the two sides' limits is that of H = max(h_i, h_j).  Where the group is a few h wide, c^2 1e5 is ~1e-8 h^2
+// and the limit is the old r2max 1.0001 to 2e-5 of r^2; the pad grows only with the group's width.
+__device__ __forceinline__ float pair_pad(const float* lo, const float* hi) {
+  const float c = 4.1e-7f * 0.5f * fmaxf(fmaxf(hi[0] - lo[0], hi[1] - lo[1]), hi[2] - lo[2]);
+  return __fmul_ru(1.0001e5f, c * c);
+}
+// r2maxif of the density prefilter: b^2 (1 + 1e-9) (the FP64 limit's margin) rounded up, then the 1e-4 for the fmaf sum
+__device__ __forceinline__ float density_bound(double h, double gd) {
+  const double b = walk_bound(h, gd);
+  return __double2float_ru(b * b * (1.0 + 1e-9)) * 1.0001f;
+}
 
 // dynamic shared memory layout: [tables: 2*(nq+1) doubles][per warp: tile 8*WALK_TILE doubles][per warp: stack+cq]
 template <bool HITER>
@@ -416,7 +457,7 @@ k_density(int n_groups, const int2* __restrict__ groups, DevParams P, DensityArr
     if (!HITER) {
       op.active = live; op.inv_h = 1.0 / hi; op.r2max = 4.0 * hi * hi * (1.0 + 1e-9); op.accW = 0.0; op.accB = 0.0;
       op.g_r2max = warp_max(live ? op.r2max : 0.0);
-      op.r2maxif = __double2float_ru(op.r2max) * 1.0001f;
+      op.r2maxif = density_bound(hi, group_half_width(op.gplo, op.gphi));
       op.list_begin(chunk);
       neighbour_walk(op, groups, chunk, box, bi, stack, cq);
       op.list_end();
@@ -455,7 +496,7 @@ k_density(int n_groups, const int2* __restrict__ groups, DevParams P, DensityArr
         op.active = iter; op.inv_h = 1.0 / hi; op.r2max = 4.0 * hi * hi * (1.0 + 1e-9); op.accW = 0.0; op.accB = 0.0;
         op.g_r2max = warp_max(iter ? op.r2max : 0.0);
         if (iter) old_len = hi;
-        op.r2maxif = __double2float_ru(op.r2max) * 1.0001f;
+        op.r2maxif = density_bound(hi, group_half_width(op.gplo, op.gphi));
         neighbour_walk(op, groups, chunk, box, bi, stack, cq);
         if (iter) {
           const double n3 = P.pi_norm * ((hi * hi) * hi), n4 = P.pi_norm * ((hi * hi) * (hi * hi));
@@ -490,7 +531,7 @@ struct ForceArrays {
 };
 #define FORCE_FIELDS 18
 #define FORCE_TG_FIELDS 19
-#define FORCE_WARP_DOUBLES (FORCE_FIELDS * WALK_TILE + FORCE_TG_FIELDS * 32 + 5 * PAIR_WIN + PAIR_WIN / 4 + 2 * WALK_TILE)   // tile + targets + results + hit list + float4 tile
+#define FORCE_WARP_DOUBLES (FORCE_FIELDS * WALK_TILE + FORCE_TG_FIELDS * 32 + 5 * PAIR_WIN + PAIR_WIN / 4 + 2 * WALK_TILE + 2)   // tile + targets + results + hit list + float4 tile + the group's pair_pad
 
 struct ForceOp {
   static const bool SYMMETRIC = true;
@@ -549,12 +590,12 @@ struct ForceOp {
     tid[s] = A.id[j];
     const double r2max_j = (fabs(A.por2[j] + A.c[j]) < INFINITY) ? 4.0 * hj * hj * (1.0 + 1e-9) : INFINITY;
     ft[s] = make_float4((float)(t[0 * WALK_TILE + s] - g0x), (float)(t[1 * WALK_TILE + s] - g0y), (float)(t[2 * WALK_TILE + s] - g0z),
-                        __double2float_ru(r2max_j));
+                        __fmaf_ru(__double2float_ru(r2max_j), 1.00012f, reinterpret_cast<const float*>(ft + WALK_TILE)[0]));
   }
   __device__ __forceinline__ void consume(int count) {
-    // Prefilter, lane = target, FP32: |x_i - x_j|^2 against max(r2max_i, r2max_j) with a 1e-4 margin that covers the
-    // float rounding of the group-relative coordinates (|coordinate| is a few h: error ~1e-6 of the limit).  It only
-    // ever drops pairs whose every term is an exact zero; the reference's own membership test (FP64, F:351-354 |
+    // Prefilter, lane = target, FP32: |x_i - x_j|^2 against the larger of the two sides' limits (pair_pad), which
+    // bounds the square of b = 2H + 4e-7 (gd + 2H), H = max(h_i, h_j) (walk_bound), the float distance of any pair
+    // with a non-zero term (r <= 2H).  It only ever drops pairs whose every term is an exact zero; the reference's own membership test (FP64, F:351-354 |
     // V:380-383) and the exact distance cull run in the lane = pair phase on the survivors.  With the exact pair
     // counter on, every staged source is a candidate.
     unsigned mask = 0;
@@ -566,11 +607,33 @@ struct ForceOp {
           const float4 sj = ft[k];
           const float dx = xif - sj.x, dy = yif - sj.y, dz = zif - sj.z;
           const float r2 = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
-          const bool far = r2 > fmaxf(r2maxif, sj.w) * 1.0001f;
+          const bool far = r2 > fmaxf(r2maxif, sj.w);
           mask |= (far ? 0u : 1u) << k;
         }
       }
     }
+#ifdef SCREEN_AUDIT
+    if (live && !count_all) {            // every staged source the screen dropped: the lane = pair phase's FP64 decision
+      const double* g = tg + (threadIdx.x & 31);
+      const int idi_ = (int)g[18 * 32];
+      unsigned bad = 0;
+      for (int k = 0; k < count; ++k) {
+        if ((mask >> k) & 1u) continue;
+        const int idj = tid[k];
+        const bool lt = idj < idi_;
+        const double xj = t[0 * WALK_TILE + k], yj = t[1 * WALK_TILE + k], zj = t[2 * WALK_TILE + k];
+        const double px = lt ? g[0 * 32] : xj, py = lt ? g[1 * 32] : yj, pz = lt ? g[2 * 32] : zj;
+        const double cx = lt ? t[13 * WALK_TILE + k] : g[13 * 32], cy = lt ? t[14 * WALK_TILE + k] : g[14 * 32], cz = lt ? t[15 * WALK_TILE + k] : g[15 * 32];
+        const double R = lt ? t[16 * WALK_TILE + k] : g[16 * 32];
+        const bool in = (idj != idi_) & (fabs(px - cx) < R) & (fabs(py - cy) < R) & (fabs(pz - cz) < R);
+        const double dx = g[0 * 32] - xj, dy = g[1 * 32] - yj, dz = g[2 * 32] - zj;
+        const double hj_ = t[7 * WALK_TILE + k];
+        const double r2max_j = (fabs(t[12 * WALK_TILE + k] + t[10 * WALK_TILE + k]) < INFINITY) ? 4.0 * hj_ * hj_ * (1.0 + 1e-9) : INFINITY;
+        bad += (in & !(dx * dx + dy * dy + dz * dz > fmax(g[17 * 32], r2max_j))) ? 1u : 0u;
+      }
+      if (bad) atomicAdd(&screen_audit[1], (unsigned long long)bad);
+    }
+#endif
     // Compact the hits (target lane, tile slot) of the whole warp and evaluate them with lane = pair: the
     // ~95 FP64 instructions of a pair run with every lane busy however unevenly a tile's sources fall among
     // the targets.  Each target then adds its own terms in tile order (F:383-391, own side; deterministic).
@@ -726,7 +789,12 @@ k_force(int n_groups, const int2* __restrict__ groups, DevParams P, ForceArrays 
       g[13 * 32] = A.lcx[ii]; g[14 * 32] = A.lcy[ii]; g[15 * 32] = A.lcz[ii]; g[16 * 32] = A.reach[ii]; g[17 * 32] = r2max; g[18 * 32] = (double)A.id[ii];
     }
     op.g0x = 0.5 * ((double)g.plo[0] + (double)g.phi[0]); op.g0y = 0.5 * ((double)g.plo[1] + (double)g.phi[1]); op.g0z = 0.5 * ((double)g.plo[2] + (double)g.phi[2]);
-    op.xif = (float)(op.xi - op.g0x); op.yif = (float)(op.yi - op.g0y); op.zif = (float)(op.zi - op.g0z); op.r2maxif = __double2float_ru(r2max);
+    op.xif = (float)(op.xi - op.g0x); op.yif = (float)(op.yi - op.g0y); op.zif = (float)(op.zi - op.g0z);
+    {
+      const float pad = pair_pad(op.gplo, op.gphi);          // kept in shared memory (after the float tile) for stage()
+      if (lane == 0) reinterpret_cast<float*>(op.ft + WALK_TILE)[0] = pad;
+      op.r2maxif = __fmaf_ru(__double2float_ru(r2max), 1.00012f, pad);
+    }
     op.g_r2max = warp_max(live ? r2max : 0.0); op.count_all = count_all != 0;
     op.ax = op.ay = op.az = op.ud = op.ad = 0.0; op.pairs = 0;
     __syncwarp();

@@ -1,7 +1,10 @@
 """Worker of tests/test_multi_gpu.py: ONE rank of an N-rank engine run, in its own process (the way bench.py and a
 production host run it: one process per rank, CUDA-IPC peers).  Not a test module.
 
-  python tests/_mp_rank.py RANK WORLD COMM DEVICE MODE STEPS OUT.npz [UID_HEX | SHM_NAME] [N] [DOMAINS]
+  python tests/_mp_rank.py RANK WORLD COMM DEVICE MODE STEPS OUT.npz [UID_HEX | SHM_NAME] [N] [DOMAINS] [EXTRA] [ICS] [CASE.npz]
+
+CASE.npz: run this input instead of the disc (`params` bytes and the in_* gas and sink columns, as tests/_cases.load_golden
+reads them); DOMAINS still sets the decomposition.
 
 COMM = nccl (needs one GPU per rank) | host (shared-memory collectives: ranks may share a device).
 """
@@ -33,7 +36,12 @@ def main():
     domains = int(sys.argv[10]) if len(sys.argv) > 10 else 0
     from summersph_b200.engine import Engine, SphError
     from summersph_b200.state import GAS_FIELDS
-    p, b, s = case(mode, n, domains)
+    if len(sys.argv) > 13 and sys.argv[13] != "-":
+        from _cases import load_golden
+        _, p, b, s = load_golden(os.path.splitext(os.path.abspath(sys.argv[13]))[0])
+        p = p.copy(decomposition=domains)
+    else:
+        p, b, s = case(mode, n, domains)
     with Engine(p, device=device) as e:
         if world > 1:
             if comm == "nccl":

@@ -29,7 +29,7 @@ def _ngpu():
         return 0
 
 
-def run_ranks(tmp_path, tag, world, comm, mode, steps=3, env_extra=None, n=60_000, domains=0, extra="-", ics="-"):
+def run_ranks(tmp_path, tag, world, comm, mode, steps=3, env_extra=None, n=60_000, domains=0, extra="-", ics="-", case="-"):
     """Launch `world` worker processes; returns the list of result dicts (one per rank)."""
     token = ""
     if world > 1:
@@ -48,7 +48,7 @@ def run_ranks(tmp_path, tag, world, comm, mode, steps=3, env_extra=None, n=60_00
         out = str(tmp_path / f"{tag}_r{r}.npz")
         dev = r if comm == "nccl" else 0
         outs.append(out)
-        procs.append(subprocess.Popen([sys.executable, WORKER, str(r), str(world), comm, str(dev), str(mode), str(steps), out, token or "-", str(n), str(domains), extra, ics],
+        procs.append(subprocess.Popen([sys.executable, WORKER, str(r), str(world), comm, str(dev), str(mode), str(steps), out, token or "-", str(n), str(domains), extra, ics, case],
                                       env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
     logs = []
     for p in procs:
