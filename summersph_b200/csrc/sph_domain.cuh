@@ -145,11 +145,10 @@ __global__ void k_dd_top_contrib(int ncell, const DDCell* __restrict__ cells, in
 }
 
 // ---- what decides "near this domain": the 8-ary BVH over the OWN walk groups (level 0 = the exported group boxes in
-// c->bvh, upper levels in a private array), walked per query with early exit.  A chunk of a Morton range can span a whole
+// c->bvh, upper levels in a private array that bi.off[l >= 1] indexes), walked per query with early exit.  A chunk of a Morton range can span a whole
 // parent cell, so a fixed handful of chunk boxes selected most of the other domain; the group boxes themselves are tight.
-struct DDBvh { int nlev; int off[12]; int cnt[12]; };
 template <class PRED>
-__device__ __forceinline__ bool dd_bvh_any(const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const DDBvh& bi, PRED pred) {
+__device__ __forceinline__ bool dd_bvh_any(const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const BvhInfo& bi, PRED pred) {
   int stack[112]; int sn = 0;                                    // <= 32 top boxes + 7 net pushes per level
   const int top = bi.nlev - 1;
   const BvhBox* tb = top == 0 ? lvl0 : upper + bi.off[top];
@@ -170,7 +169,7 @@ __device__ __forceinline__ bool dd_bvh_any(const BvhBox* __restrict__ lvl0, cons
 // every run of this rank whatever path the classification takes, so its children are never read.
 struct DDLetEntry { int slot, owner, rchild, nchild; };    // patch wnodes[slot].child; children live at peer `owner`, index rchild
 struct DDPeerNodes { const WNode* wn[DD_MAX_RANKS]; };
-__device__ __forceinline__ bool dd_may_open(const WNode& w, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const DDBvh& bi, double theta2) {
+__device__ __forceinline__ bool dd_may_open(const WNode& w, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const BvhInfo& bi, double theta2) {
   const double s2 = w.size * w.size * (1.0 + 1e-4);
   const double cx = w.cx, cy = w.cy, cz = w.cz;
   return dd_bvh_any(lvl0, upper, bi, [&](const BvhBox& q) {
@@ -186,7 +185,7 @@ __device__ __forceinline__ bool dd_may_open(const WNode& w, const BvhBox* __rest
 // are in flight together.  ctl: [0] cursor, [1] overflow flag, [2 + level] frontier counts.
 __global__ void k_dd_let_level(const DDLetEntry* __restrict__ fin, const int* __restrict__ n_in, DDLetEntry* __restrict__ fout, int* n_out,
                                int fcap, int* cursor, int let_end, int* overflow, const __grid_constant__ DDPeerNodes peers,
-                               WNode* __restrict__ wn, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const __grid_constant__ DDBvh bi, double theta2) {
+                               WNode* __restrict__ wn, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const __grid_constant__ BvhInfo bi, double theta2) {
   const int n = *n_in < fcap ? *n_in : fcap;
   const int k = threadIdx.x & 7, lane = threadIdx.x & 31;
   const unsigned gmask = 0xffu << (lane & 24);
@@ -214,7 +213,7 @@ __global__ void k_dd_let_level(const DDLetEntry* __restrict__ fin, const int* __
 }
 // top-region entries whose children live on a peer: decide whether this domain may open them (frontier of level 0)
 __global__ void k_dd_let_seed(int n_cand, const DDLetEntry* __restrict__ cand, DDLetEntry* __restrict__ fout, int* n_out,
-                              const WNode* __restrict__ wn, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const __grid_constant__ DDBvh bi, double theta2) {
+                              const WNode* __restrict__ wn, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper, const __grid_constant__ BvhInfo bi, double theta2) {
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n_cand) return;
   const DDLetEntry e = cand[t];
@@ -228,7 +227,7 @@ struct DDPeerGroups { int ng[DD_MAX_RANKS]; int goff[DD_MAX_RANKS + 1]; const in
 // domain (x_i inside Box(j), F:443 | V:479) or its position box meets a reach box (x_j inside Box(i), the pair loop's
 // other direction).  A superset is harmless: the walks keep their exact tests.
 __global__ void k_dd_halo_mark(const __grid_constant__ DDPeerGroups pg, const BvhBox* __restrict__ lvl0, const BvhBox* __restrict__ upper,
-                               const __grid_constant__ DDBvh bi, unsigned char* __restrict__ flag, int* __restrict__ hsize) {
+                               const __grid_constant__ BvhInfo bi, unsigned char* __restrict__ flag, int* __restrict__ hsize) {
   const int G = blockIdx.x * blockDim.x + threadIdx.x;
   if (G == pg.goff[DD_MAX_RANKS]) hsize[G] = 0;                  // the scan's total lands here
   if (G >= pg.goff[DD_MAX_RANKS]) return;

@@ -124,7 +124,7 @@ struct sph_ctx {
   bool dd = false; int64_t n_global = 0; int n_halo = 0, ng_own = 0, ng_halo = 0;
   uint64_t* key_alloc[2] = {}; int* perm_alloc[2] = {};          // the allocations behind key[] / perm[] (which swap)
   uint64_t *dd_samples = nullptr, *dd_split = nullptr; long long* dd_counts = nullptr; int* dd_sendoff = nullptr; uint64_t* dd_segkeys = nullptr; std::vector<WNode> dd_top_host; std::vector<int> dd_top_part;
-  DDCell* dd_cells = nullptr; DDContrib* dd_contrib = nullptr; BvhBox* dd_obvh = nullptr; size_t dd_obvh_cap = 0; DDBvh dd_ob; int* dd_let_ctl = nullptr; double* dd_create8 = nullptr; unsigned long long* dd_cand = nullptr;
+  DDCell* dd_cells = nullptr; DDContrib* dd_contrib = nullptr; BvhBox* dd_obvh = nullptr; size_t dd_obvh_cap = 0; BvhInfo dd_ob; int* dd_let_ctl = nullptr; double* dd_create8 = nullptr; unsigned long long* dd_cand = nullptr;
   bool dd_fields_pending = false; cudaEvent_t let_done = nullptr; bool let_pending = false; double* let_flag = nullptr; std::vector<DDLetEntry> dd_cand_host;
   DDLetEntry* dd_let_f[2] = {}; int dd_let_fcap = 0, dd_let_begin = 0, dd_let_end = 0, dd_let_used = 0, dd_top_n = 0;
   unsigned char* dd_halo_flag = nullptr; int *dd_halo_list = nullptr, *dd_halo_size = nullptr, *dd_halo_poff = nullptr; size_t dd_halo_cap = 0;
@@ -140,6 +140,8 @@ namespace {
 #define LAUNCH(kern, grid, block, smem, ...) do { kern<<<(grid), (block), (smem), c->stream>>>(__VA_ARGS__); ++c->launches; } while (0)
 
 inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
+// boxes of the levels above n0 level-0 boxes of the 8-ary BVH (bvh_levels): below n0 / 7, plus one partial box per level
+inline size_t bvh_upper_boxes(int64_t n0) { return (size_t)(n0 / 7 + 64); }
 
 StateArrays state_of(sph_ctx* c, int which) {
   double** s = c->st[which];
@@ -193,7 +195,7 @@ int ensure_capacity(sph_ctx* c, int64_t n) {
     DA(c->wnodes, (size_t)c->dd_let_end);
     DA(c->dd_let_f[0], c->dd_let_fcap); DA(c->dd_let_f[1], c->dd_let_fcap);
     DA(c->dd_acc_key, cap); DA(c->dd_acc_rec, cap);
-    c->bvh_cap = (size_t)(cap + cap / 7 + 64) * 5 / 4; DA(c->bvh, c->bvh_cap);
+    c->bvh_cap = (cap + bvh_upper_boxes(cap)) * 5 / 4; DA(c->bvh, c->bvh_cap);
   } else DA(c->wnodes, 2 * cap);
   DA(c->wcount, 2 * cap); DA(c->wstart, 2 * cap); DA(c->widx, 2 * cap);
   DA(c->keep, cap); DA(c->pos, cap); DA(c->stage_d, cap); DA(c->stage_d2, cap);
@@ -210,6 +212,14 @@ int ensure_capacity(sph_ctx* c, int64_t n) {
   if (cudaMalloc(&c->cub_tmp, c->cub_bytes) != cudaSuccess) { c->err = "cudaMalloc(cub temp)"; cudaGetLastError(); return SPH_ERR_OOM; }
   c->cap = cap;
   c->p2p_stale = true;
+  return SPH_OK;
+}
+
+// grow the CUB temp storage to at least `bytes`
+int cub_reserve(sph_ctx* c, size_t bytes) {
+  if (bytes + 256 <= c->cub_bytes) return SPH_OK;
+  c->cub_bytes = bytes + 256; if (c->cub_tmp) cudaFree(c->cub_tmp); c->cub_tmp = nullptr;
+  if (cudaMalloc(&c->cub_tmp, c->cub_bytes) != cudaSuccess) { c->err = "cudaMalloc(cub temp)"; return SPH_ERR_OOM; }
   return SPH_OK;
 }
 
@@ -509,6 +519,101 @@ int id_ranks(sph_ctx* c, int n, const int* id, int* cnt, int* off, int* pos) {
   return SPH_OK;
 }
 
+// Root cube (F:803-808) and descent keys of the n current particles.  The replicated form's ranks all hold every particle
+// and find the same cube alone; under domains the extrema are all-reduced (min / max are exact: the same cube as one rank's).
+int root_and_keys(sph_ctx* c, int n, uint64_t* key_lo) {
+  const int T = 256;
+  StateArrays s = state_of(c, c->cur);
+  const int nb = std::max(1, std::min(cdiv(n, T), c->n_partial));
+  LAUNCH(k_bbox_partial, nb, T, 0, n, s.x, s.y, s.z, c->partial);
+  LAUNCH(k_bbox_final, 1, 32, 0, nb, c->partial, c->root);
+  if (c->dd) {
+    LAUNCH(k_dd_box_pack, 1, 32, 0, c->root, c->partial);            // [mn, -mx] so that one MIN all-reduce merges both
+    { int r_ = coll_allreduce(c, c->stream, c->partial, 6, NC_FLOAT64, NC_MIN); if (r_) return r_; }
+    LAUNCH(k_dd_box_unpack, 1, 32, 0, c->partial);
+    LAUNCH(k_bbox_final, 1, 32, 0, 1, c->partial, c->root);
+  }
+  LAUNCH(k_keys, cdiv(std::max(n, 1), T), T, 0, n, s.x, s.y, s.z, c->root, c->dp.lmax, c->key[0], key_lo, c->perm[0]);
+  return SPH_OK;
+}
+
+// stable radix sort of (key[0], perm[0]) by the single-word key; the sorted pair ends up in key[0] / perm[0]
+int sort_keys(sph_ctx* c, int n) {
+  size_t bytes = c->cub_bytes;
+  cub::DoubleBuffer<uint64_t> dk(c->key[0], c->key[1]); cub::DoubleBuffer<int> dv(c->perm[0], c->perm[1]);
+  CK(cub::DeviceRadixSort::SortPairs(c->cub_tmp, bytes, dk, dv, n, 0, 63, c->stream));
+  if (dk.Current() != c->key[0]) std::swap(c->key[0], c->key[1]);
+  if (dv.Current() != c->perm[0]) std::swap(c->perm[0], c->perm[1]);
+  return SPH_OK;
+}
+
+// The local octree over the n sorted particles, in two halves so that a caller can act on a key collision in between.
+// Leaf cells, then the internal-node count and the key-collision flag on the host.  has_prev / kprev, has_next / knext:
+// under domains, the boundary keys of the neighbouring domains (k_leaf); zeros otherwise.
+int octree_leaves(sph_ctx* c, int n, const uint64_t* klo, int has_prev, uint64_t kprev, int has_next, uint64_t knext, int* nn, int* key_err) {
+  const int T = 256;
+  StateArrays s = state_of(c, c->cur);
+  { int r_ = flush_late(c, LF_H); if (r_) return r_; }
+  LAUNCH(k_leaf, cdiv(n, T), T, 0, n, c->key[0], klo, s.h, c->root, c->dp, c->level, c->lcx, c->lcy, c->lcz, c->reach, &c->sc->err, has_prev, kprev, has_next, knext);
+  LAUNCH(k_oct_nodes<false>, cdiv(n, T), T, 0, n, c->key[0], klo, c->dp.lmax, c->root, c->cnt, c->off, 0, c->nodes, c->node_part, c->node_count);
+  CK(cudaMemsetAsync(c->cnt + n, 0, sizeof(int), c->stream));
+  size_t bytes = c->cub_bytes;
+  CK(cub::DeviceScan::ExclusiveSum(c->cub_tmp, bytes, c->cnt, c->off, n + 1, c->stream));
+  // node count is needed on the host for launch sizes of the per-node passes
+  readback(c, c->h_rb, c->off + n, sizeof(int));
+  readback(c, c->h_rb + 1, &c->sc->err, sizeof(int));
+  CK(cudaStreamSynchronize(c->stream));
+  *nn = n + c->h_rb[0]; *key_err = c->h_rb[1];
+  return SPH_OK;
+}
+// The nn nodes (preorder), their links, walk-layout slots and sums (k_oct_finalize is left to the caller), then the walk
+// groups: cell-aligned buckets, their sizes in gsize, their first particles in gfirst and their count in d_nsel (device).
+int octree_nodes(sph_ctx* c, int n, int nn, const uint64_t* klo) {
+  const int T = 256;
+  StateArrays s = state_of(c, c->cur);
+  c->counts.n_nodes = nn;
+  LAUNCH(k_oct_nodes<true>, cdiv(n, T), T, 0, n, c->key[0], klo, c->dp.lmax, c->root, c->cnt, c->off, nn, c->nodes, c->node_part, c->node_count);
+  LAUNCH(k_oct_link, cdiv(nn, T), T, 0, nn, c->nodes, c->node_part, c->parent, c->nchild, c->wcount);
+  size_t bytes = c->cub_bytes;
+  CK(cub::DeviceScan::ExclusiveSum(c->cub_tmp, bytes, c->wcount, c->wstart, nn, c->stream));
+  CK(cudaMemsetAsync(c->widx, 0xff, sizeof(int) * (size_t)nn, c->stream));
+  LAUNCH(k_oct_widx, cdiv(nn, T), T, 0, nn, c->nodes, c->wcount, c->wstart, c->widx);
+  CK(cudaMemsetAsync(c->arrive, 0, sizeof(int) * (size_t)nn, c->stream));
+  { int r_ = flush_late(c, LF_M | LF_H); if (r_) return r_; }
+  LAUNCH(k_oct_up, cdiv(n, T), T, 0, n, c->off, c->cnt, s.x, s.y, s.z, s.m, s.h, c->level, c->root, c->nodes, c->parent, c->nchild, c->arrive);
+  CK(cudaMemsetAsync(c->gsize, 0, sizeof(int) * (size_t)n, c->stream));
+  LAUNCH(k_group_mark, cdiv(nn, T), T, 0, nn, c->nodes, c->node_part, c->node_count, c->gsize);
+  bytes = c->cub_bytes;
+  CK(cub::DeviceSelect::Flagged(c->cub_tmp, bytes, cub::CountingInputIterator<int>(0), c->gsize, c->gfirst, c->d_nsel, n, c->stream));
+  return SPH_OK;
+}
+
+// The implicit 8-ary BVH above n0 level-0 boxes at lvl0: every level boxes SPH_BVH_FAN boxes of the one below, up to a
+// level of at most 32.  Level l >= 1 is written at upper + bi.off[l], the first of them at upper + off1.
+void bvh_levels(sph_ctx* c, const BvhBox* lvl0, int n0, BvhBox* upper, int off1, BvhInfo& bi) {
+  const int T = 256;
+  bi.off[0] = 0; bi.cnt[0] = n0;
+  int l = 0;
+  for (int off = off1; bi.cnt[l] > 32; ++l) {
+    const int np = cdiv(bi.cnt[l], SPH_BVH_FAN);
+    bi.off[l + 1] = off; bi.cnt[l + 1] = np;
+    LAUNCH(k_bvh_up, cdiv(np, T), T, 0, bi.cnt[l], l == 0 ? lvl0 : upper + bi.off[l], upper + off);
+    off += np;
+  }
+  bi.nlev = l + 1;
+}
+
+// global segment table of the sink sums, nst segments: [segment][sink][3].  Outside the domain form it is peer-mapped,
+// so a new allocation voids the mapping (the first exchange after a build maps it again)
+int sink_seg_reserve(sph_ctx* c, int nst) {
+  const int nsk = std::max(c->n_sink, 1);
+  if ((size_t)nst * nsk * 3 > c->sink_seg_cap) {
+    c->sink_seg_cap = (size_t)(nst + nst / 8 + 64) * (nsk + 1) * 3;
+    DA(c->sink_seg, c->sink_seg_cap); if (!c->dd) c->p2p_stale = true;
+  }
+  return SPH_OK;
+}
+
 #include "sph_domain_host.inl"
 
 // Single-word (63-bit, 21-level) keys are the fast path.  If two particles share a full key while the
@@ -521,10 +626,9 @@ int refresh_tree(sph_ctx* c) {
   if (c->dp.variable_h) {
     StateArrays s = state_of(c, c->cur);
     LAUNCH(k_refresh_reach, cdiv(n, T), T, 0, n, s.h, c->level, c->root, c->dp, c->reach);
-    const BvhInfo& bi = c->bi;
-    LAUNCH(k_bvh_leaf, cdiv((int64_t)bi.cnt[0] * 32, T), T, 0, bi.cnt[0], c->groups, s.x, s.y, s.z, c->lcx, c->lcy, c->lcz, c->reach, c->bvh);
-    for (int l = 0; l + 1 < bi.nlev; ++l)
-      LAUNCH(k_bvh_up, cdiv(bi.cnt[l + 1], T), T, 0, bi.cnt[l], c->bvh + bi.off[l], c->bvh + bi.off[l + 1]);
+    const int ng = c->n_groups;
+    LAUNCH(k_bvh_leaf, cdiv((int64_t)ng * 32, T), T, 0, ng, c->groups, s.x, s.y, s.z, c->lcx, c->lcy, c->lcz, c->reach, c->bvh);
+    bvh_levels(c, c->bvh, ng, c->bvh, ng, c->bi);
   }
   stage_end(c);
   return SPH_OK;
@@ -554,30 +658,19 @@ int build_tree_impl(sph_ctx* c, bool* retry_two_word) {
   if (c->two_word && !c->key_lo[0]) { for (int b = 0; b < 2; ++b) DA(c->key_lo[b], c->cap); }
   if (c->late_pending && c->late_permuted) { int r_ = flush_late(c, LF_ALL); if (r_) return r_; }      // a second re-order (two-word retry) takes complete columns
   stage_begin(c, ST_KEYS);
-  {
-    StateArrays s = state_of(c, c->cur);
-    int nb = std::min(cdiv(n, T), c->n_partial);
-    LAUNCH(k_bbox_partial, nb, T, 0, n, s.x, s.y, s.z, c->partial);
-    // multi-GPU: particles are replicated, every rank sees the same box (no exchange needed)
-    LAUNCH(k_bbox_final, 1, 32, 0, nb, c->partial, c->root);
-    LAUNCH(k_keys, cdiv(n, T), T, 0, n, s.x, s.y, s.z, c->root, c->dp.lmax, c->key[0], c->two_word ? c->key_lo[0] : nullptr, c->perm[0]);
-  }
+  { int r_ = root_and_keys(c, n, c->two_word ? c->key_lo[0] : nullptr); if (r_) return r_; }
   stage_end(c);
   stage_begin(c, ST_SORT);
   {
-    size_t bytes = c->cub_bytes;
     if (c->two_word) {     // stable LSD order: low word first
+      size_t bytes = c->cub_bytes;
       cub::DoubleBuffer<uint64_t> dl(c->key_lo[0], c->key_lo[1]); cub::DoubleBuffer<int> dv(c->perm[0], c->perm[1]);
       CK(cub::DeviceRadixSort::SortPairs(c->cub_tmp, bytes, dl, dv, n, 0, 63, c->stream));
       if (dv.Current() != c->perm[0]) std::swap(c->perm[0], c->perm[1]);
       LAUNCH(k_gather_u64, cdiv(n, T), T, 0, n, c->perm[0], c->key[0], c->key[1]);
       std::swap(c->key[0], c->key[1]);
-      bytes = c->cub_bytes;
     }
-    cub::DoubleBuffer<uint64_t> dk(c->key[0], c->key[1]); cub::DoubleBuffer<int> dv(c->perm[0], c->perm[1]);
-    CK(cub::DeviceRadixSort::SortPairs(c->cub_tmp, bytes, dk, dv, n, 0, 63, c->stream));
-    if (dk.Current() != c->key[0]) { std::swap(c->key[0], c->key[1]); }
-    if (dv.Current() != c->perm[0]) { std::swap(c->perm[0], c->perm[1]); }
+    { int r_ = sort_keys(c, n); if (r_) return r_; }
     PermuteArgs pa;
     for (int f = 0; f < 10; ++f) { pa.src[f] = c->st[c->cur][f]; pa.dst[f] = c->st[c->cur ^ 1][f]; }
     pa.id_src = c->id[c->cur]; pa.id_dst = c->id[c->cur ^ 1];
@@ -595,65 +688,29 @@ int build_tree_impl(sph_ctx* c, bool* retry_two_word) {
   stage_end(c);
   stage_begin(c, ST_TREE);
   {
-    StateArrays s = state_of(c, c->cur);
     const uint64_t* klo = c->two_word ? c->key_lo[0] : nullptr;
-    { int r_ = flush_late(c, LF_H); if (r_) return r_; }
-    LAUNCH(k_leaf, cdiv(n, T), T, 0, n, c->key[0], klo, s.h, c->root, c->dp, c->level, c->lcx, c->lcy, c->lcz, c->reach, &c->sc->err);
-    // octree
-    LAUNCH(k_oct_nodes<false>, cdiv(n, T), T, 0, n, c->key[0], klo, c->dp.lmax, c->root, c->cnt, c->off, 0, c->nodes, c->node_part, c->node_count);
-    CK(cudaMemsetAsync(c->cnt + n, 0, sizeof(int), c->stream));
-    size_t bytes = c->cub_bytes;
-    CK(cub::DeviceScan::ExclusiveSum(c->cub_tmp, bytes, c->cnt, c->off, n + 1, c->stream));
-    // node count is needed on the host for launch sizes of the per-node passes
-    readback(c, c->h_rb, c->off + n, sizeof(int));
-    readback(c, c->h_rb + 1, &c->sc->err, sizeof(int));
-    CK(cudaStreamSynchronize(c->stream));
-    const int n_int = c->h_rb[0], key_err = c->h_rb[1];
+    int nn = 0, key_err = 0;
+    { int r_ = octree_leaves(c, n, klo, 0, 0, 0, 0, &nn, &key_err); if (r_) return r_; }
     if (key_err && !c->two_word) {            // a 63-bit key collision: redo this build with two-word keys
       CK(cudaMemsetAsync(&c->sc->err, 0, sizeof(int), c->stream));
       stage_end(c);
       *retry_two_word = true;
       return SPH_OK;
     }
-    const int nn = n + n_int;
-    c->counts.n_nodes = nn;
-    LAUNCH(k_oct_nodes<true>, cdiv(n, T), T, 0, n, c->key[0], klo, c->dp.lmax, c->root, c->cnt, c->off, nn, c->nodes, c->node_part, c->node_count);
-    LAUNCH(k_oct_link, cdiv(nn, T), T, 0, nn, c->nodes, c->node_part, c->parent, c->nchild, c->wcount);
-    bytes = c->cub_bytes;
-    CK(cub::DeviceScan::ExclusiveSum(c->cub_tmp, bytes, c->wcount, c->wstart, nn, c->stream));
-    CK(cudaMemsetAsync(c->widx, 0xff, sizeof(int) * (size_t)nn, c->stream));
-    LAUNCH(k_oct_widx, cdiv(nn, T), T, 0, nn, c->nodes, c->wcount, c->wstart, c->widx);
-    CK(cudaMemsetAsync(c->arrive, 0, sizeof(int) * (size_t)nn, c->stream));
-    { int r_ = flush_late(c, LF_M | LF_H); if (r_) return r_; }
-    LAUNCH(k_oct_up, cdiv(n, T), T, 0, n, c->off, c->cnt, s.x, s.y, s.z, s.m, s.h, c->level, c->root, c->nodes, c->parent, c->nchild, c->arrive);
+    { int r_ = octree_nodes(c, n, nn, klo); if (r_) return r_; }
     LAUNCH(k_oct_finalize, cdiv(nn, T), T, 0, nn, c->nodes, c->wcount, c->wstart, c->widx, c->wnodes);
-    // walk groups (cell-aligned buckets) and the implicit 8-ary BVH over them
-    CK(cudaMemsetAsync(c->gsize, 0, sizeof(int) * (size_t)n, c->stream));
-    LAUNCH(k_group_mark, cdiv(nn, T), T, 0, nn, c->nodes, c->node_part, c->node_count, c->gsize);
-    bytes = c->cub_bytes;
-    CK(cub::DeviceSelect::Flagged(c->cub_tmp, bytes, cub::CountingInputIterator<int>(0), c->gsize, c->gfirst, c->d_nsel, n, c->stream));
     readback(c, c->h_rb, c->d_nsel, sizeof(int));
     CK(cudaStreamSynchronize(c->stream));
     const int ng = c->h_rb[0];
     c->n_groups = ng;
-    if ((size_t)ng + ng / 7 + 64 > c->bvh_cap) { c->bvh_cap = (size_t)(ng + ng / 7 + 64) * 5 / 4; DA(c->bvh, c->bvh_cap); }
+    if (ng + bvh_upper_boxes(ng) > c->bvh_cap) { c->bvh_cap = (ng + bvh_upper_boxes(ng)) * 5 / 4; DA(c->bvh, c->bvh_cap); }
     LAUNCH(k_group_pack, cdiv(ng, T), T, 0, ng, c->gfirst, c->gsize, c->groups);
-    BvhInfo& bi = c->bi;
-    int cntl = ng, offl = 0, l = 0;
-    bi.off[0] = 0; bi.cnt[0] = cntl;
-    LAUNCH(k_bvh_leaf, cdiv((int64_t)cntl * 32, T), T, 0, ng, c->groups, s.x, s.y, s.z, c->lcx, c->lcy, c->lcz, c->reach, c->bvh);
-    while (cntl > 32) {
-      int np = cdiv(cntl, SPH_BVH_FAN);
-      bi.off[l + 1] = offl + cntl; bi.cnt[l + 1] = np;
-      LAUNCH(k_bvh_up, cdiv(np, T), T, 0, cntl, c->bvh + offl, c->bvh + offl + cntl);
-      offl += cntl; cntl = np; ++l;
-    }
-    bi.nlev = l + 1;
+    StateArrays s = state_of(c, c->cur);
+    LAUNCH(k_bvh_leaf, cdiv((int64_t)ng * 32, T), T, 0, ng, c->groups, s.x, s.y, s.z, c->lcx, c->lcy, c->lcz, c->reach, c->bvh);
+    bvh_levels(c, c->bvh, ng, c->bvh, ng, c->bi);
     { int r_ = compute_slices(c); if (r_) return r_; }
-    {   // global segment table of the sink sums: sized here so that the peer mapping (first exchange = density) sees it
-      const int nst = cdiv(c->n_groups, GRAV_SEG), nsk = std::max(c->n_sink, 1);
-      if ((size_t)nst * nsk * 3 > c->sink_seg_cap) { c->sink_seg_cap = (size_t)(nst + nst / 8 + 64) * (nsk + 1) * 3; DA(c->sink_seg, c->sink_seg_cap); c->p2p_stale = true; }
-    }
+    // sized here so that the peer mapping (first exchange = density) sees it
+    { int r_ = sink_seg_reserve(c, cdiv(ng, GRAV_SEG)); if (r_) return r_; }
   }
   stage_end(c);
   c->tree_valid = true; c->pos_moved = false;
@@ -848,11 +905,8 @@ int run_gravity(sph_ctx* c, int do_grav, int do_sinks) {
 #endif
   // sink side of the gas terms: per-segment folds -> exchange of the rows -> one fixed fold over all segments (rank-count independent)
   {
-    const int nst = cdiv(c->dd ? c->g1 : c->n_groups, GRAV_SEG), nsk = std::max(c->n_sink, 1);
-    if ((size_t)nst * nsk * 3 > c->sink_seg_cap) {
-      c->sink_seg_cap = (size_t)(nst + nst / 8 + 64) * (nsk + 1) * 3;
-      DA(c->sink_seg, c->sink_seg_cap); if (!c->dd) c->p2p_stale = true;
-    }
+    const int nst = cdiv(c->dd ? c->g1 : c->n_groups, GRAV_SEG);
+    { int r_ = sink_seg_reserve(c, nst); if (r_) return r_; }
     if (do_sinks && nseg > 0 && c->g1 > c->g0)
       LAUNCH(k_sink_seg_fold, cdiv((int64_t)nseg * c->n_sink * 3, 128), 128, 0, nseg, seg0, c->n_sink, c->seg_off, c->sink_partial, c->sink_seg);
     stage_end(c);
@@ -1156,21 +1210,13 @@ int interp_scratch(sph_ctx* c, size_t cap) {
 int interp_bvh(sph_ctx* c, int ng, int n_src) {
   const int T = 256;
   if ((size_t)n_src > c->ip_reach_cap) { c->ip_reach_cap = 0; DA(c->ip_reach, (size_t)c->cap); c->ip_reach_cap = (size_t)c->cap; }
-  if ((size_t)ng + ng / 7 + 64 > c->ip_bvh_cap) { c->ip_bvh_cap = 0; const size_t cap = (size_t)(ng + ng / 7 + 64) * 5 / 4; DA(c->ip_bvh, cap); c->ip_bvh_cap = cap; }
-  BvhInfo& bi = c->ip_bi;
-  bi.nlev = 1; bi.off[0] = 0; bi.cnt[0] = ng;
-  if (ng == 0) return SPH_OK;
-  StateArrays s = state_of(c, c->cur);
-  LAUNCH(k_interp_reach, cdiv(n_src, T), T, 0, n_src, s.h, c->dp.variable_h, c->dp.h_fixed, c->ip_reach);
-  LAUNCH(k_bvh_leaf, cdiv((int64_t)ng * 32, T), T, 0, ng, c->groups, s.x, s.y, s.z, s.x, s.y, s.z, c->ip_reach, c->ip_bvh);
-  int cntl = ng, offl = 0, l = 0;
-  while (cntl > 32) {
-    const int np = cdiv(cntl, SPH_BVH_FAN);
-    bi.off[l + 1] = offl + cntl; bi.cnt[l + 1] = np;
-    LAUNCH(k_bvh_up, cdiv(np, T), T, 0, cntl, c->ip_bvh + offl, c->ip_bvh + offl + cntl);
-    offl += cntl; cntl = np; ++l;
+  if (ng + bvh_upper_boxes(ng) > c->ip_bvh_cap) { c->ip_bvh_cap = 0; const size_t cap = (ng + bvh_upper_boxes(ng)) * 5 / 4; DA(c->ip_bvh, cap); c->ip_bvh_cap = cap; }
+  if (ng > 0) {
+    StateArrays s = state_of(c, c->cur);
+    LAUNCH(k_interp_reach, cdiv(n_src, T), T, 0, n_src, s.h, c->dp.variable_h, c->dp.h_fixed, c->ip_reach);
+    LAUNCH(k_bvh_leaf, cdiv((int64_t)ng * 32, T), T, 0, ng, c->groups, s.x, s.y, s.z, s.x, s.y, s.z, c->ip_reach, c->ip_bvh);
   }
-  bi.nlev = l + 1;
+  bvh_levels(c, c->ip_bvh, ng, c->ip_bvh, ng, c->ip_bi);
   return SPH_OK;
 }
 
