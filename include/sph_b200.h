@@ -347,6 +347,38 @@ int sph_column_density(sph_ctx* ctx, int32_t axis, double u0, double u1, double 
 int sph_interpolate(sph_ctx* ctx, int64_t n_points, const double* px, const double* py, const double* pz,
                     double* out, int32_t n_out);
 
+/* The gravitational potential and acceleration at n_points caller-given points (px, py, pz: host arrays): rotation
+ * curves, mid-plane potential maps, what a test particle would feel.  Point k is treated as a gas particle of smoothing
+ * length h_k (h = NULL: h_k = h_fixed for every point) placed at x_k that adds nothing to the tree; the result is what
+ * particle_gravforce_one (F:264-290 | V:285-311) and sink_gravforces (F:559-591 | V:691-726) give that particle:
+ *   accepted nodes: the reference's opening test, size / dist < theta or the node has no children (theta = 0.5, or
+ *             params.theta under theta_override), dist = sqrt(|x - COM|^2 + soft), soft = 0.001 h_fixed
+ *             (0.001 h_k with SPH_FLAG_SOFT_USES_HI); kernel length h' = h_fixed (fixed h, F:280) | h_k (variable h, V:301)
+ *   out[c * n_points + k], c = 0 .. n_out - 1 (n_out <= SPH_GRAVAT_COUNT):
+ *     0  phi_gas = G sum over the accepted nodes of M phi(dist / h') / h', phi = the softened potential of sph_conserved
+ *        (-1/q beyond q = 2).  No node is left out: a point on a particle includes that particle's own softened term,
+ *        whereas sph_conserved's E_gg leaves a particle's own leaf out.
+ *     1..3  g_gas = -G sum M g(dist / h') (x - COM) / dist^3, the reference's term; at a particle's own position with its
+ *        own h this is the gravity pass's gas-gas acceleration of that particle (its own leaf has direction 0)
+ *     4  phi_sink = -G sum_s m_s / |x - x_s|, unsoftened (F:572), over the sinks with m_s > 0 and |x - x_s| > 0 (the
+ *        zero-mass dummy sink and a point exactly on a sink add nothing)
+ *     5..7  g_sink = -G sum_s m_s (x - x_s) / |x - x_s|^3 over the same sinks
+ *     8  the number of nodes the walk accepted, as a double (the reference's grav_accepted for such a particle)
+ * SPH_ERR_ARG: a NULL px / py / pz / out, n_out outside 1..SPH_GRAVAT_COUNT, n_points < 0, a non-finite coordinate or
+ * (h given) an h_k that is not finite and positive; SPH_ERR_STATE: no gas uploaded; n_points = 0 is a no-op.
+ * Builds the tree of the current positions if the context holds none (kept for the next evaluation, like
+ * sph_interpolate) and changes nothing a later step reads: the stored far-field sums and near-pair records,
+ * sph_counters, sph_stage_times, sph_far_reuse_count and the state arrays (ax / ay / az included) are left as they
+ * were, and the sinks feel no back-reaction.  A repeated call returns the same bits, and a permutation of the points
+ * the permuted output.  Replicated multi-GPU form: every rank computes locally and returns the same bits.  Under
+ * decomposition = 1 the call is collective: every rank passes the same points and h (checked: count and a hash of the
+ * bits; a mismatch is SPH_ERR_ARG on every rank); each rank adds the tree nodes it owns (a node straddling ranks is
+ * added on rank 0), the gas columns are summed over the ranks and the sink columns are computed after that, so every
+ * rank returns the same bits: `accepted` equal to the single-rank count, the values equal up to summation order. */
+#define SPH_GRAVAT_COUNT 9
+int sph_gravity_at(sph_ctx* ctx, int64_t n_points, const double* px, const double* py, const double* pz,
+                   const double* h, double* out, int32_t n_out);
+
 #ifdef __cplusplus
 }
 #endif

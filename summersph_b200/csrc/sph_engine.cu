@@ -27,6 +27,7 @@
 #include "sph_conserved.cuh"
 #include "sph_image.cuh"
 #include "sph_interp.cuh"
+#include "sph_gravat.cuh"
 #include "sph_domain.cuh"
 #include "sph_ics.cuh"
 
@@ -120,10 +121,13 @@ struct sph_ctx {
   double* ip_reach = nullptr; size_t ip_reach_cap = 0; BvhBox* ip_bvh = nullptr; size_t ip_bvh_cap = 0; BvhInfo ip_bi;
   double *ip_pts = nullptr, *ip_raw = nullptr, *ip_bpart = nullptr; uint64_t *ip_key[2] = {}, *ip_tie[2] = {}; int* ip_idx[2] = {}; RootBox* ip_rb = nullptr;
   void* ip_cub = nullptr; size_t ip_cub_bytes = 0; size_t ip_cap = 0;
+  // sph_gravity_at: the points (x, y, z, h) and the output columns of one chunk (sorted by the sph_interpolate scratch), the top-slot owners
+  double *ga_q = nullptr, *ga_raw = nullptr; size_t ga_cap = 0; int* ga_owner = nullptr;
   // ---- Morton-domain decomposition (sph_domain.cuh / sph_domain_host.inl); in this mode n = own particles, cap = own + halo capacity
   bool dd = false; int64_t n_global = 0; int n_halo = 0, ng_own = 0, ng_halo = 0;
   uint64_t* key_alloc[2] = {}; int* perm_alloc[2] = {};          // the allocations behind key[] / perm[] (which swap)
   uint64_t *dd_samples = nullptr, *dd_split = nullptr; long long* dd_counts = nullptr; int* dd_sendoff = nullptr; uint64_t* dd_segkeys = nullptr; std::vector<WNode> dd_top_host; std::vector<int> dd_top_part;
+  std::vector<int> dd_top_owner;      // per top slot: the rank holding the complete node, -1 for a cell straddling ranks (sph_gravity_at)
   DDCell* dd_cells = nullptr; DDContrib* dd_contrib = nullptr; BvhBox* dd_obvh = nullptr; size_t dd_obvh_cap = 0; BvhInfo dd_ob; int* dd_let_ctl = nullptr; double* dd_create8 = nullptr; unsigned long long* dd_cand = nullptr;
   bool dd_fields_pending = false; cudaEvent_t let_done = nullptr; bool let_pending = false; double* let_flag = nullptr; std::vector<DDLetEntry> dd_cand_host;
   DDLetEntry* dd_let_f[2] = {}; int dd_let_fcap = 0, dd_let_begin = 0, dd_let_end = 0, dd_let_used = 0, dd_top_n = 0;
@@ -1220,12 +1224,11 @@ int interp_bvh(sph_ctx* c, int ng, int n_src) {
   return SPH_OK;
 }
 
-// One chunk of points [off, off + nc): sort, walk, (domains) sum the ranks' raw columns, finish, copy out.
-int interp_chunk(sph_ctx* c, int64_t off, int nc, const double* px, const double* py, const double* pz, int64_t n_points,
-                 double* out, int n_out, bool reduce) {
+// Points [off, off + nc) to the device (pts + k * ip_cap) and their order: sorted by k_interp_keys' Morton key, ties by the
+// coordinate-bit hash, so the sorted sequence does not depend on the caller's order.  *perm[i] = the chunk index of the i-th.
+int interp_sort(sph_ctx* c, int64_t off, int nc, const double* px, const double* py, const double* pz, double* pts, int** perm_out) {
   const int T = 256;
   const size_t cap = c->ip_cap;
-  double* pts = c->ip_pts;
   const double* src[3] = {px, py, pz};
   for (int k = 0; k < 3; ++k) CK(cudaMemcpyAsync(pts + (size_t)k * cap, src[k] + off, (size_t)nc * 8, cudaMemcpyHostToDevice, c->stream));
   const int nb = std::min(cdiv(nc, T), c->n_partial);
@@ -1244,6 +1247,18 @@ int interp_chunk(sph_ctx* c, int64_t off, int nc, const double* px, const double
     CK(cub::DeviceRadixSort::SortPairs(c->ip_cub, bytes, dk, dp, nc, 0, 63, c->stream));
     perm = dp.Current();
   }
+  *perm_out = perm;
+  return SPH_OK;
+}
+
+// One chunk of points [off, off + nc): sort, walk, (domains) sum the ranks' raw columns, finish, copy out.
+int interp_chunk(sph_ctx* c, int64_t off, int nc, const double* px, const double* py, const double* pz, int64_t n_points,
+                 double* out, int n_out, bool reduce) {
+  const int T = 256;
+  const size_t cap = c->ip_cap;
+  double* pts = c->ip_pts;
+  int* perm;
+  { int r = interp_sort(c, off, nc, px, py, pz, pts, &perm); if (r) return r; }
   const int ng = c->ip_bi.cnt[0];
   StateArrays s = state_of(c, c->cur);
   InterpArrays A{s.x, s.y, s.z, s.vx, s.vy, s.vz, s.u, s.m, s.alpha, s.h, c->ip_reach};
@@ -1258,6 +1273,31 @@ int interp_chunk(sph_ctx* c, int64_t off, int nc, const double* px, const double
     for (size_t o = 0; o < tot; o += chunk) { int r = coll_allreduce(c, c->stream, raw + o, std::min(chunk, tot - o), NC_FLOAT64, NC_SUM); if (r) return r; }
   }
   LAUNCH(k_interp_finish, cdiv(nc, T), T, 0, nc, raw);
+  for (int k = 0; k < n_out; ++k)
+    CK(cudaMemcpyAsync(out + (size_t)k * n_points + off, raw + (size_t)k * nc, (size_t)nc * 8, cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return SPH_OK;
+}
+
+// ---- sph_gravity_at (sph_gravat.cuh) ------------------------------------------------------------------------------
+// One chunk of points [off, off + nc): sort, walk (one thread per point), (domains) sum the ranks' gas columns, sinks, copy out.
+int gravat_chunk(sph_ctx* c, int64_t off, int nc, const double* px, const double* py, const double* pz, const double* h,
+                 int64_t n_points, double* out, int n_out, bool reduce) {
+  const int T = 256;
+  const size_t cap = c->ip_cap;
+  double* q = c->ga_q;
+  int* perm;
+  { int r = interp_sort(c, off, nc, px, py, pz, q, &perm); if (r) return r; }
+  if (h) CK(cudaMemcpyAsync(q + 3 * cap, h + off, (size_t)nc * 8, cudaMemcpyHostToDevice, c->stream));
+  double* raw = c->ga_raw;
+  const int rank = c->dd ? c->rank : 0;
+  LAUNCH(k_gravity_at, cdiv(nc, GRAVAT_THREADS), GRAVAT_THREADS, 0, nc, q, cap, h ? 1 : 0, perm, c->dp, c->wnodes, c->d_gt,
+         c->dd ? DD_TOP_CAP : 0, c->ga_owner, rank, raw);
+  if (reduce) {      // NCCL: one all-reduce; the host communicator's all-gather carries at most SPH_HC_SLOT bytes per rank
+    const size_t tot = (size_t)GRAVAT_RAW * nc, chunk = c->hc ? SPH_HC_SLOT / 8 : tot;
+    for (size_t o = 0; o < tot; o += chunk) { int r = coll_allreduce(c, c->stream, raw + o, std::min(chunk, tot - o), NC_FLOAT64, NC_SUM); if (r) return r; }
+  }
+  LAUNCH(k_gravity_at_sinks, cdiv(nc, T), T, 0, nc, q, cap, c->dp, c->n_sink, c->S, raw);
   for (int k = 0; k < n_out; ++k)
     CK(cudaMemcpyAsync(out + (size_t)k * n_points + off, raw + (size_t)k * nc, (size_t)nc * 8, cudaMemcpyDeviceToHost, c->stream));
   CK(cudaStreamSynchronize(c->stream));
@@ -1375,6 +1415,7 @@ int sph_destroy(sph_ctx* c) {
   F(c->dd_accg_key[0]); F(c->dd_accg_key[1]); F(c->dd_accg_idx[0]); F(c->dd_accg_idx[1]); F(c->dd_accg_rec); F(c->dd_gid); F(c->dd_gpos); F(c->dd_gcnt); F(c->dd_goff); F(c->dd_gstage);
   F(c->cons_partial); F(c->cons_out); F(c->cons_wpart); F(c->img_table); F(c->sink_spin);
   F(c->ip_reach); F(c->ip_bvh); F(c->ip_pts); F(c->ip_raw); F(c->ip_bpart); F(c->ip_rb); F(c->ip_cub);
+  F(c->ga_q); F(c->ga_raw); F(c->ga_owner);
   for (int b = 0; b < 2; ++b) { F(c->ip_key[b]); F(c->ip_tie[b]); F(c->ip_idx[b]); }
   F(c->far_fx); F(c->far_fy); F(c->far_fz); F(c->far_hc2); F(c->far_ctr); F(c->far_list); F(c->far_cnt); F(c->far_ovf); F(c->d_same); F(c->sink_land);
   F(c->arrive); F(c->cnt); F(c->off); F(c->root); F(c->partial); F(c->cub_tmp); F(c->d_wt); F(c->d_dwt); F(c->d_gt);
@@ -2114,6 +2155,70 @@ int sph_interpolate(sph_ctx* c, int64_t n_points, const double* px, const double
   for (int64_t off = 0; off < n_points; off += SPH_INTERP_CHUNK) {      // the chunks depend on n_points only: the same on every rank
     const int nc = (int)std::min<int64_t>(SPH_INTERP_CHUNK, n_points - off);
     int r = interp_chunk(c, off, nc, px, py, pz, n_points, out, n_out, coll);
+    if (r) return r;
+  }
+  CK(cudaGetLastError());
+  return SPH_OK;
+}
+
+int sph_gravity_at(sph_ctx* c, int64_t n_points, const double* px, const double* py, const double* pz, const double* h,
+                   double* out, int32_t n_out) {
+  if (!c) return SPH_ERR_ARG;
+  cudaSetDevice(c->device);
+  const bool coll = c->dd && c->n_ranks > 1;      // domains: every rank walks the nodes it owns for the same points, the gas sums are added
+  std::string why;
+  if (!px || !py || !pz || !out) why = "null pointer";
+  else if (n_out < 1 || n_out > SPH_GRAVAT_COUNT) why = "n_out must be 1.." + std::to_string(SPH_GRAVAT_COUNT);
+  else if (n_points < 0) why = "n_points < 0";
+  uint64_t hash = 0;
+  if (why.empty()) {
+    const double* col[4] = {px, py, pz, h};
+    for (int64_t i = 0; i < n_points && why.empty(); ++i)
+      for (int k = 0; k < (h ? 4 : 3); ++k) {
+        const double v = col[k][i];
+        if (!std::isfinite(v)) { why = k < 3 ? "non-finite coordinate" : "h must be finite and positive"; break; }
+        if (k == 3 && !(v > 0.0)) { why = "h must be finite and positive"; break; }
+        if (coll) { uint64_t b; std::memcpy(&b, &v, 8); hash = mix64(hash ^ b); }
+      }
+  }
+  if (coll) {      // the ranks compare their points (count, hash of the coordinate and h bits, n_out) and argument checks
+    struct Fp { int64_t n; uint64_t h; int32_t n_out, bad; };
+    Fp mine = {n_points, hash ^ (h ? 1ull : 0ull), n_out, why.empty() ? 0 : 1}, all[DD_MAX_RANKS];
+    { int r = dd_allgather_host(c, &mine, sizeof(Fp), all); if (r) return r; }
+    for (int q = 0; q < c->n_ranks && why.empty(); ++q) {
+      if (all[q].bad) why = "rank " + std::to_string(q) + " passed invalid arguments";
+      else if (all[q].n != mine.n || all[q].h != mine.h || all[q].n_out != mine.n_out) why = "the ranks passed different points (the call is collective: every rank passes the same points)";
+    }
+  }
+  if (!why.empty()) { c->err = "sph_gravity_at: " + why; return SPH_ERR_ARG; }
+  if ((c->dd ? c->n_global : c->n) <= 0) { c->err = "no particles uploaded"; return SPH_ERR_STATE; }
+  if (n_points == 0) return SPH_OK;
+  double keep_ms[ST_COUNT]; std::memcpy(keep_ms, c->stage_ms, sizeof(keep_ms));
+  if (!(c->tree_valid && !c->pos_moved)) {        // the octree of the current positions (kept for the next evaluation); domains: migration, halo, LET
+    int r = build_tree(c); if (r) return r;
+  }
+  int code = interp_scratch(c, (size_t)std::min<int64_t>(n_points, SPH_INTERP_CHUNK));
+  if (!code && c->ga_cap < c->ip_cap) {
+    c->ga_cap = 0;
+    code = dalloc(c, &c->ga_q, 4 * c->ip_cap);
+    if (!code) code = dalloc(c, &c->ga_raw, (size_t)GRAVAT_COLS * c->ip_cap);
+    if (!code) c->ga_cap = c->ip_cap;
+  }
+  if (!code && c->dd) {
+    if (!c->ga_owner) code = dalloc(c, &c->ga_owner, DD_TOP_CAP);
+    if (!code) CK(cudaMemcpyAsync(c->ga_owner, c->dd_top_owner.data(), c->dd_top_owner.size() * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+    if (c->let_pending) { CK(cudaStreamWaitEvent(c->stream, c->let_done, 0)); c->let_pending = false; }      // no LET slot is read, but its pull writes the layout
+  }
+  CK(cudaMemcpyAsync(c->h_sc, c->sc, sizeof(SimScalars), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  stage_collect(c, false);                        // a tree build here is not part of any step's stage times
+  std::memcpy(c->stage_ms, keep_ms, sizeof(keep_ms));
+  if (!code) code = check_device_error(c);        // key-depth error of a tree built here
+  if (coll) { int r = dd_agree(c, code, "sph_gravity_at"); if (r) return r; }
+  else if (code) return code;
+  for (int64_t off = 0; off < n_points; off += SPH_INTERP_CHUNK) {      // the chunks depend on n_points only: the same on every rank
+    const int nc = (int)std::min<int64_t>(SPH_INTERP_CHUNK, n_points - off);
+    int r = gravat_chunk(c, off, nc, px, py, pz, h, n_points, out, n_out, coll);
     if (r) return r;
   }
   CK(cudaGetLastError());

@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("SPH_B200_LIB") or os.path.join(_HERE, "libsph_b200.so
 _LIB = None
 
 INTERP = ("rho", "vx", "vy", "vz", "u", "alpha", "count")      # the SPH_INTERP_COUNT output columns of sph_interpolate
+GRAVAT = ("phi_gas", "gx_gas", "gy_gas", "gz_gas", "phi_sink", "gx_sink", "gy_sink", "gz_sink", "accepted")   # SPH_GRAVAT_COUNT columns of sph_gravity_at
 STAGES = ("keys", "sort", "tree", "density", "gravity", "sph", "integrate", "h_iter", "cull", "comm", "halo", "let", "migrate", "gravity_near")
 
 
@@ -80,6 +81,7 @@ def load_library(path=None):
     lib.sph_download_sink_spin.argtypes = [vp, vp, vp, vp]
     lib.sph_column_density.argtypes = [vp, i32, dbl, dbl, dbl, dbl, i32, i32, vp]
     lib.sph_interpolate.argtypes = [vp, i64, vp, vp, vp, vp, i32]
+    lib.sph_gravity_at.argtypes = [vp, i64, vp, vp, vp, vp, vp, i32]
     if path is None:
         _LIB = lib
     return lib
@@ -327,6 +329,21 @@ class Engine:
         out = np.zeros(max(int(n_out), 0) * m)
         self._ck(self._l.sph_interpolate(self._c, m, *[_p(c) for c in cols], _p(out), int(n_out)))
         return {k: out[i * m:(i + 1) * m] for i, k in enumerate(INTERP[:n_out])}
+
+    def gravity_at(self, points, h=None, n_out=len(GRAVAT)):
+        """The gravitational potential and acceleration at the rows of `points` ((M, 3): x, y, z), computed on the device
+        (`sph_gravity_at`): dict of length-M arrays {phi_gas, gx_gas, gy_gas, gz_gas, phi_sink, gx_sink, gy_sink, gz_sink,
+        accepted} truncated to the first `n_out`.  Each point is treated as a gas particle of smoothing length `h` (length-M
+        array; None: h_fixed) that adds nothing to the tree: the gas part is the reference's Barnes-Hut sum over the nodes
+        it would accept, the sink part the unsoftened direct sum.  Collective under the Morton domains: every rank passes
+        the same points and h."""
+        pts = np.asarray(points, dtype=np.float64).reshape(-1, 3)
+        m = len(pts)
+        cols = [np.ascontiguousarray(pts[:, k]) for k in range(3)]
+        hh = None if h is None else np.ascontiguousarray(np.broadcast_to(np.asarray(h, dtype=np.float64), (m,)))
+        out = np.zeros(max(int(n_out), 0) * m)
+        self._ck(self._l.sph_gravity_at(self._c, m, *[_p(c) for c in cols], _p(hh), _p(out), int(n_out)))
+        return {k: out[i * m:(i + 1) * m] for i, k in enumerate(GRAVAT[:n_out])}
 
     def group_count(self):
         return int(self._l.sph_group_count(self._c))
