@@ -83,7 +83,7 @@ struct sph_ctx {
   int* h_rb = nullptr;                                      // pinned scratch for readback(): 16 ints
   int resident_check = 1; int64_t resident_hits = 0; int* d_same = nullptr; double* sink_land = nullptr;      // upload_impl: "is this the state I hold?"
   WalkCounters* ctr = nullptr; WalkCounters* h_ctr = nullptr; int* work = nullptr;
-  unsigned char* keep = nullptr; unsigned long long* acc_key[2] = {}; int* acc_val[2] = {}; int* d_nsel = nullptr;
+  unsigned char* keep = nullptr; unsigned long long* acc_key[2] = {}; int* acc_val[2] = {}; int64_t acc_cap = 0; int* d_nsel = nullptr;   // accretion list (ensure_acc_capacity)
   int* pos = nullptr;           // ascending-number position of each sorted particle (downloads)
   double* stage_d = nullptr; double* stage_d2 = nullptr; int stage_flip = 0;   // device staging for ordered downloads
   bool tree_valid = false; bool pos_moved = true; int tree_reuse = 1; int use_lists = 1; int fused_push = 1; int nl_exact = 0; int exact_counters = 0;   // pos_moved: positions / particle set changed since the last build
@@ -180,12 +180,33 @@ template <class T> int dalloc(sph_ctx* c, T** p, size_t count) {
 }
 #define DA(ptr, count) do { int r_ = dalloc(c, &(ptr), (size_t)(count)); if (r_) return r_; } while (0)
 
+int cub_reserve(sph_ctx* c, size_t bytes);
+
+// The accretion list of k_flags: one (sink, particle) entry for every sink whose radius holds the particle (each sink
+// accretes on its own, F:484-556 | V:616-688), so with overlapping sinks it can hold more entries than there are
+// particles.  Grown to at least `want` entries, never below `cap` (the domain re-order borrows acc_key[0] / acc_val[0]
+// as merge scratch); under domains the exported records (dd_acc_key / dd_acc_rec, k_dd_acc_records) are as long.  The CUB
+// temp storage is checked every time: ensure_capacity re-sizes it for the particle count alone.
+int ensure_acc_capacity(sph_ctx* c, int64_t want) {
+  if (want > c->acc_cap || (c->dd && !c->dd_acc_key)) {
+    const int64_t cap = std::max(want, c->acc_cap);
+    c->acc_cap = 0;
+    for (int b = 0; b < 2; ++b) { DA(c->acc_key[b], cap); DA(c->acc_val[b], cap); }
+    if (c->dd) { DA(c->dd_acc_key, cap); DA(c->dd_acc_rec, cap); c->p2p_stale = true; }
+    c->acc_cap = cap;
+  }
+  size_t b1 = 0;
+  cub::DoubleBuffer<unsigned long long> dk(c->acc_key[0], c->acc_key[1]); cub::DoubleBuffer<int> dv(c->acc_val[0], c->acc_val[1]);
+  cub::DeviceRadixSort::SortPairs(nullptr, b1, dk, dv, (int)c->acc_cap, 0, 64, c->stream);
+  return cub_reserve(c, b1);
+}
+
 int ensure_capacity(sph_ctx* c, int64_t n) {
   if (n <= c->cap) return SPH_OK;
   const int64_t cap = n + n / 64 + 1024;
   c->cap = 0; c->tree_valid = false; c->pos_moved = true; c->p2p_stale = true;      // a failed grow must not leave the old capacity standing over freed arrays
   for (int b = 0; b < 2; ++b) if (c->key_lo[b]) { cudaFree(c->key_lo[b]); c->key_lo[b] = nullptr; }
-  for (int b = 0; b < 2; ++b) { for (int f = 0; f < 10; ++f) DA(c->st[b][f], cap); DA(c->id[b], cap); DA(c->key[b], cap); DA(c->perm[b], cap); DA(c->acc_key[b], cap); DA(c->acc_val[b], cap); }
+  for (int b = 0; b < 2; ++b) { for (int f = 0; f < 10; ++f) DA(c->st[b][f], cap); DA(c->id[b], cap); DA(c->key[b], cap); DA(c->perm[b], cap); }
   for (int b = 0; b < 2; ++b) { c->key_alloc[b] = c->key[b]; c->perm_alloc[b] = c->perm[b]; }
   DA(c->rho, cap); DA(c->omega, cap); DA(c->prs, cap); DA(c->cs, cap); DA(c->por2, cap);
   DA(c->ax, cap); DA(c->ay, cap); DA(c->az, cap); DA(c->udot, cap); DA(c->adot, cap);
@@ -194,11 +215,10 @@ int ensure_capacity(sph_ctx* c, int64_t n) {
   DA(c->node_count, 2 * cap); DA(c->gsize, cap); DA(c->gfirst, cap); DA(c->groups, cap);
   DA(c->nodes, 2 * cap); DA(c->node_part, 2 * cap); DA(c->parent, 2 * cap); DA(c->nchild, 2 * cap); DA(c->arrive, 2 * cap);
   DA(c->cnt, cap + 1); DA(c->off, cap + 1);
-  if (c->dd) {      // walk layout: [top tree | local tree | locally essential nodes of the peers]; accretion records; LET frontier; fixed BVH capacity (exported)
+  if (c->dd) {      // walk layout: [top tree | local tree | locally essential nodes of the peers]; LET frontier; fixed BVH capacity (exported)
     c->dd_let_begin = DD_TOP_CAP + (int)(2 * cap); c->dd_let_end = c->dd_let_begin + (int)cap; c->dd_let_fcap = (int)std::max<int64_t>(cap / 4, 65536);
     DA(c->wnodes, (size_t)c->dd_let_end);
     DA(c->dd_let_f[0], c->dd_let_fcap); DA(c->dd_let_f[1], c->dd_let_fcap);
-    DA(c->dd_acc_key, cap); DA(c->dd_acc_rec, cap);
     c->bvh_cap = (cap + bvh_upper_boxes(cap)) * 5 / 4; DA(c->bvh, c->bvh_cap);
   } else DA(c->wnodes, 2 * cap);
   DA(c->wcount, 2 * cap); DA(c->wstart, 2 * cap); DA(c->widx, 2 * cap);
@@ -214,6 +234,7 @@ int ensure_capacity(sph_ctx* c, int64_t n) {
   c->cub_bytes = std::max(std::max(std::max(b1, b4), std::max(b2, b3)), b5) + 256;
   if (c->cub_tmp) { cudaFree(c->cub_tmp); c->cub_tmp = nullptr; }
   if (cudaMalloc(&c->cub_tmp, c->cub_bytes) != cudaSuccess) { c->err = "cudaMalloc(cub temp)"; cudaGetLastError(); return SPH_ERR_OOM; }
+  { int r_ = ensure_acc_capacity(c, cap); if (r_) return r_; }
   c->cap = cap;
   c->p2p_stale = true;
   return SPH_OK;
@@ -1077,14 +1098,22 @@ int step(sph_ctx* c) {
   }
   stage_begin(c, ST_CULL);
   LAUNCH(k_any_sink_mass, 1, 32, 0, c->S, c->sc);                             // F:919
-  LAUNCH(k_flags, cdiv(n, T), T, 0, n, c->dp, state_of(c, c->cur), c->key[0], c->two_word ? c->key_lo[0] : nullptr, c->level, c->lcx, c->lcy, c->lcz, c->reach, c->root,
-         c->S, c->sc, c->keep, c->acc_key[0], c->acc_val[0], (int)c->cap);
-  readback(c, c->h_sc, c->sc, sizeof(SimScalars));
-  CK(cudaStreamSynchronize(c->stream));
-  if ((r = check_device_error(c))) return r;
-  if (c->h_sc->n_accreted > (int)c->cap) {      // k_flags already dropped the particles: never truncate silently
-    c->err = "accretion list overflow: " + std::to_string(c->h_sc->n_accreted) + " (sink, particle) entries, capacity " + std::to_string((long long)c->cap);
-    return SPH_ERR_STATE;
+  auto flags = [&]() -> int {
+    LAUNCH(k_flags, cdiv(n, T), T, 0, n, c->dp, state_of(c, c->cur), c->key[0], c->two_word ? c->key_lo[0] : nullptr, c->level, c->lcx, c->lcy, c->lcz, c->reach, c->root,
+           c->S, c->sc, c->keep, c->acc_key[0], c->acc_val[0], (int)c->acc_cap);
+    readback(c, c->h_sc, c->sc, sizeof(SimScalars));
+    CK(cudaStreamSynchronize(c->stream));
+    return check_device_error(c);
+  };
+  if ((r = flags())) return r;
+  // k_flags counts every (sink, particle) entry but stores only the first acc_cap: a particle inside several sinks' radii is
+  // accreted by each of them, so the list can outgrow the particle count.  Then grow it and flag again - k_flags reads
+  // only the state, the tree and the sinks and rewrites keep[] for every row, so the second pass is the first one whole
+  if (c->h_sc->n_accreted > c->acc_cap) {
+    const int64_t want = (int64_t)c->h_sc->n_accreted;
+    if ((r = ensure_acc_capacity(c, want + want / 8 + 1024))) return r;
+    CK(cudaMemsetAsync(&c->sc->n_removed, 0, sizeof(int) * 2, c->stream));      // n_removed, n_accreted
+    if ((r = flags())) return r;
   }
   int n_acc = c->h_sc->n_accreted;
   int n_removed_global = c->h_sc->n_removed;
