@@ -257,6 +257,13 @@ int64_t sph_group_count(sph_ctx* ctx);
  * a full walk, summed in another order.  SPH_B200_NO_FAR_REUSE=1 (environment, read in sph_create) turns it off. */
 int64_t sph_far_reuse_count(sph_ctx* ctx);
 
+/* Walk runs (32 Morton-consecutive particles) that the last full gravity walk storing far sums flagged because some
+ * particle of the run had more near terms than the records hold per particle (128; SPH_B200_FAR_SLOTS=n, read in
+ * sph_create, sets another count): the next near-only evaluation serves those runs by the near-only walk instead of the
+ * records.  0 before the first such walk; a full walk that stores nothing (exact counters, first step on a new state)
+ * sets it back to 0. */
+int64_t sph_far_overflow_runs(sph_ctx* ctx);
+
 /* A host that owns the state between steps (upload, loop body, download - the reference's own loop keeps bodies(:) /
  * sinks(:) on the host side, SUMMER_SPH.f90:879-929) hands back exactly what it was given.  sph_upload / sph_step_host
  * therefore compare the incoming x y z m h and sinks bitwise, on the device, with the state the context holds (rows by

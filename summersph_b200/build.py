@@ -28,14 +28,20 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
+def nvcc_command(out, extra=()):
+    """The nvcc command line that builds the engine into `out`; `extra`: more flags, e.g. ["-DSCREEN_AUDIT"] for a variant."""
+    cmd = [nvcc_path()] + NVCC_FLAGS + list(extra) + ["-o", out] + [os.path.join(CSRC, s) for s in SOURCES] + ["-ldl"]
+    if os.path.exists("/usr/bin/g++"):
+        cmd[1:1] = ["-ccbin", "/usr/bin/g++"]
+    return cmd
+
+
 def build_extension(force=False, verbose=False):
     """Compile the engine for sm_100a. Returns the path of the shared library."""
     if not force and not needs_build():
         return SO
-    cmd = [nvcc_path()] + NVCC_FLAGS + ["-o", SO] + [os.path.join(CSRC, s) for s in SOURCES] + ["-ldl"]
+    cmd = nvcc_command(SO)
     env = dict(os.environ)
-    if os.path.exists("/usr/bin/g++"):
-        cmd[1:1] = ["-ccbin", "/usr/bin/g++"]
     res = subprocess.run(cmd, capture_output=True, text=True, env=env)
     log = res.stdout + res.stderr
     with open(os.path.join(HERE, "csrc", "build.log"), "w") as f:

@@ -1998,6 +1998,7 @@ int sph_stage_times(sph_ctx* c, double* ms, int32_t n) {
 int64_t sph_launch_count(sph_ctx* c) { return c ? c->launches : 0; }
 int64_t sph_group_count(sph_ctx* c) { return c ? c->n_groups : 0; }
 int64_t sph_far_reuse_count(sph_ctx* c) { return c ? c->far_count : 0; }
+int64_t sph_far_overflow_runs(sph_ctx* c) { return c ? c->far_n_ovf : 0; }
 int64_t sph_resident_hits(sph_ctx* c) { return c ? c->resident_hits : 0; }
 int sph_set_resident_check(sph_ctx* c, int32_t on) { if (!c) return SPH_ERR_ARG; c->resident_check = on ? 1 : 0; return SPH_OK; }
 

@@ -71,6 +71,8 @@ def load_library(path=None):
     lib.sph_group_count.restype = i64
     lib.sph_far_reuse_count.argtypes = [vp]
     lib.sph_far_reuse_count.restype = i64
+    lib.sph_far_overflow_runs.argtypes = [vp]
+    lib.sph_far_overflow_runs.restype = i64
     lib.sph_resident_hits.argtypes = [vp]
     lib.sph_resident_hits.restype = i64
     lib.sph_set_resident_check.argtypes = [vp, i32]
@@ -358,3 +360,8 @@ class Engine:
     def far_reuse_count(self):
         """Gravity evaluations so far that walked only the near field on top of the stored far sums."""
         return int(self._l.sph_far_reuse_count(self._c))
+
+    def far_overflow_runs(self):
+        """Walk runs the last far-sum-storing gravity walk flagged for the near-only walk: some particle had more
+        near terms than the recorded slots (`sph_far_overflow_runs`)."""
+        return int(self._l.sph_far_overflow_runs(self._c))
